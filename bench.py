@@ -2,6 +2,7 @@
 """bench.py -- train audio-sec/sec of the CPC hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME] [--batch B]
+                    [--dump-outputs DIR]
 
 Workloads (``--workload``; the default is the one BASELINE.json's metric is quoted on):
 
@@ -23,7 +24,18 @@ trainer objects with every batch coming from pinned host memory and the loss rea
 single most expensive kernel (one entry point at one shape, timed with CUDA events inside real steps), `metrics`
 (CQT GB/s and dense-equivalent TFLOP/s, InfoNCE TFLOP/s, conv TFLOP/s by kernel family) and `cpu_baseline` (the oracle
 port of the same step on the host cores, bounded sample).  `--impl reference` times that CPU port alone (the reference is
-CPU-only Python and /root/reference does not travel to the GPU box, so kind = "port").
+CPU-only Python, so kind = "port").
+
+`--dump-outputs DIR` writes what the last timed step computed (rank 0) as float32 .npy files: loss.npy and max_score.npy
+(what the step returns) and gradients.npy (the gradient of every trainable parameter that the optimizer applies, i.e.
+averaged over ranks, flattened and concatenated in model.parameters() order). An array longer than DUMP_SAMPLE entries
+is stored as a fixed, seeded sample of DUMP_SAMPLE entries (in index order). Every timed step starts from the seeded
+initial state (see run_ours) on seeded batches, so two runs, or two builds, run with the same arguments can be compared
+output for output: one run of a build repeats another up to the rounding of a single step. Each timed step is timed
+alone with its own CUDA events, so the restore before it and any gap between steps are not timed, and each is the
+optimizer's first step. The parameters after the optimizer step are not written: a conv bias that feeds a train-mode
+batch norm has a true gradient of exactly zero, so its computed gradient is rounding noise, and Adam turns that noise
+into a step of +-lr.
 """
 import argparse
 import json
@@ -39,6 +51,7 @@ sys.path.insert(0, PKG)
 
 SR = 16000
 METRIC = "train audio-sec/sec"
+DUMP_SAMPLE = 1 << 22                                           # entries kept of a longer dumped array (16 MB in fp32)
 
 WORKLOADS = {
     "e24": {"batch": 64, "cpu_batch": 8, "visible": 60, "prediction": 16, "dtype": "f32",
@@ -69,6 +82,21 @@ def measured_peaks():
         return {"hbm": p["hbm_gbs"], "tensor_burst": p["bf16_tflops"], "tensor": p["bf16_tflops_sustained"],
                 "source": "measured"}
     return {"hbm": 6650.0, "tensor_burst": 1590.0, "tensor": 1400.0, "source": "fallback"}
+
+
+def dump_outputs(path, arrays):
+    """Write each tensor of ``arrays`` (name -> tensor) as ``path/<name>.npy`` in float32.  A tensor of more than
+    DUMP_SAMPLE entries is flattened and only the entries at DUMP_SAMPLE indices drawn with a fixed seed (kept in index
+    order) are written: the same entries on every run, so dumps of two builds line up."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().to(torch.float32).cpu()
+        if a.numel() > DUMP_SAMPLE:
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(path, name + ".npy"), a.numpy())
 
 
 class ClockSampler:
@@ -326,6 +354,13 @@ def run_ours(args):
             dist.barrier()
         torch.cuda.synchronize()
 
+    def max_over_ranks(ms):
+        if world > 1:
+            t = torch.tensor([ms], device=dev)
+            dist.all_reduce(t, op=dist.ReduceOp.MAX)
+            ms = t.item()
+        return ms
+
     def timed(fn, k):
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -334,22 +369,52 @@ def run_ours(args):
             fn(i)
         e1.record()
         barrier()
-        ms = e0.elapsed_time(e1)
-        if world > 1:
-            t = torch.tensor([ms], device=dev)
-            dist.all_reduce(t, op=dist.ReduceOp.MAX)
-            ms = t.item()
-        return ms / k
+        return max_over_ranks(e0.elapsed_time(e1)) / k
+
+    # Every timed step trains from the seeded initial state: the weights and buffers as they are now (before the warm-up
+    # steps) and a fresh optimizer state (zero moments and step count), restored on the device before the step and
+    # outside its events.  The kernels reduce with float atomics, whose order differs from run to run, and a chain of
+    # training steps amplifies such last-bit differences; from one fixed state a step does the same work as any other
+    # and computes the same result in every run, up to the rounding of that one step.
+    initial = [(t, t.detach().clone()) for m in (model, pre) if m is not None
+               for t in list(m.parameters()) + list(m.buffers())]
 
     clocks = ClockSampler(local)
     clocks.start()                                              # nvidia-smi needs a moment to deliver its first sample
     for i in range(args.warmup):
         step(dev_batches[i % 2])
     torch.cuda.synchronize()
+    opt_state = [v for st in optimizer.state.values() for v in st.values() if torch.is_tensor(v)]
+    opt_state += [g["_step_state"] for g in optimizer.param_groups if torch.is_tensor(g.get("_step_state"))]
+    state = [t for t, _ in initial] + opt_state
+    saved = [v for _, v in initial] + [torch.zeros_like(v) for v in opt_state]
+
+    def restore():
+        with torch.no_grad():
+            for t, v in zip(state, saved):
+                t.copy_(v)
     _lib.reset_launch_count()
     t_load = time.time()
-    ms_dev = timed(lambda i: step(dev_batches[i % 2]), args.steps)
+    barrier()
+    events = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
+    for i, (e0, e1) in enumerate(events):
+        restore()
+        e0.record()
+        last_out = step(dev_batches[i % 2])
+        e1.record()
+    barrier()
+    ms_dev = max_over_ranks(sum(e0.elapsed_time(e1) for e0, e1 in events)) / args.steps
     launches = launches_per_step * args.steps if graphed is not None else _lib.launch_count()
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # device copies now: the steps below overwrite the graph's static outputs and the gradients.  The graphed
+        # multi-rank step leaves the sum over ranks in .grad and lets cpc_b200.optim.Adam scale it by 1 / world; every
+        # other path leaves the average there, which is what is written.
+        params = [p for p in model.parameters() if p.requires_grad]
+        scale = 1.0 / world if graphed is not None and world > 1 and isinstance(optimizer, cpc_b200.optim.Adam) else 1.0
+        dumped = {"loss": last_out[0].clone(), "max_score": last_out[1].clone(),
+                  "gradients": scale * torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).detach()
+                                                  .reshape(-1) for p in params])}
     # K steps of ~14 ms are shorter than a few 100 ms sampling periods: keep the identical load running (untimed) until
     # ~0.6 s of it have been sampled.  The count derives from ms_dev (max over ranks), so every rank runs the same steps.
     clock_window = "timed region"
@@ -511,6 +576,8 @@ def run_ours(args):
             "kernels": top[:40]}
     if world > 1:
         line["overlap"] = getattr(graphed, "overlap_description", None)
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     emit(line)
     if world > 1:
         sys.stderr.flush()
@@ -519,8 +586,9 @@ def run_ours(args):
 
 def run_infonce_sweep(args):
     """BASELINE configs[3]: fused InfoNCE forward + backward alone.  candidates N in 128...8192, K in 4...32, E = 512; per-step
-    mode B = N, all-steps mode B = N / K; linear and softplus; regulariser 0 and 0.01.  Prints one JSON line whose `value`
-    is the best fwd+bwd TFLOP/s of the sweep (algorithmic FLOPs = 4 x forward) and whose `sweep` lists every point."""
+    mode B = N, all-steps mode B = N / K; linear and softplus; regulariser 0 and 0.01; each point timed over --steps calls.
+    Prints one JSON line whose `value` is the best fwd+bwd TFLOP/s of the sweep (algorithmic FLOPs = 4 x forward) and
+    whose `sweep` lists every point."""
     import torch
     from cpc_b200 import _lib, ops
     if not torch.cuda.is_available():
@@ -550,7 +618,7 @@ def run_infonce_sweep(args):
                     for _ in range(2):
                         once()
                     torch.cuda.synchronize()
-                    reps = 3 if n >= 4096 else 10
+                    reps = args.steps
                     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                     e0.record()
                     for _ in range(reps):
@@ -563,7 +631,7 @@ def run_infonce_sweep(args):
                                    "score": kind, "reg": reg, "ms": ms, "tflops": 4.0 * fwd / (ms * 1e-3) / 1e12})
     best = max(points, key=lambda p: p["tflops"])
     emit({"metric": "InfoNCE fused score+loss fwd+bwd TFLOP/s (sweep best)", "value": best["tflops"], "unit": "TFLOP/s",
-          "n_gpus": 1, "steps": 1, "warmup": 2, "ms_per_step": best["ms"], "higher_is_better": True, "scaling": "weak",
+          "n_gpus": 1, "steps": args.steps, "warmup": 2, "ms_per_step": best["ms"], "higher_is_better": True, "scaling": "weak",
           "vs_baseline": None, "dtype": "f32", "data": "synthetic",
           "config": {"workload": "infonce_sweep: fused InfoNCE fwd+bwd, E=512, candidates 128-8192 x K 4-32 (BASELINE configs[3])",
                      "best_point": best},
@@ -606,7 +674,13 @@ def main():
     ap.add_argument("--workload", default="e24", choices=sorted(WORKLOADS) + ["infonce_sweep"])
     ap.add_argument("--batch", type=int, default=None, help="items per GPU (default: the workload's)")
     ap.add_argument("--no-graph", action="store_true", help="submit kernels eagerly instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed training step computed to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "infonce_sweep"):
+        ap.error("--dump-outputs applies to the training-step workloads of --impl ours")
     args.warmup = max(3, args.warmup) if args.impl == "ours" else args.warmup
     if args.workload == "infonce_sweep":
         if args.impl == "reference":

@@ -1569,3 +1569,34 @@ def test_two_rank_nccl_parity(cpc):
     print(out.stdout[-3000:])
     assert out.returncode == 0, out.stdout[-3000:] + out.stderr[-3000:]
     assert "RANK_OK 0" in out.stdout and "RANK_OK 1" in out.stdout
+
+
+def test_bench_dump_outputs_of_the_last_timed_step(cpc, tmp_path):
+    """bench.py --dump-outputs: loss, max score and gradients of the last timed step as float32, under 64 MB in all.
+    Every timed step trains from the seeded initial state on batch i % 2, so the last steps of --steps 1 and --steps 3
+    (both batch 0, separate runs) agree up to the rounding of one step, and that of --steps 2 (batch 1) does not."""
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    dumps = {}
+    for steps in (1, 3, 2):
+        out_dir = tmp_path / str(steps)
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--workload", "raw_wave", "--batch", "2",
+                              "--steps", str(steps), "--warmup", "1", "--dump-outputs", str(out_dir)],
+                             capture_output=True, text=True, timeout=900)
+        assert out.returncode == 0, out.stderr[-3000:]
+        assert json.loads(out.stdout.strip().splitlines()[-1])["steps"] == steps
+        names = sorted(os.listdir(out_dir))
+        assert names == ["gradients.npy", "loss.npy", "max_score.npy"], names
+        assert sum(os.path.getsize(out_dir / n) for n in names) <= 64 << 20
+        dumps[steps] = {n[:-4]: np.load(out_dir / n) for n in names}
+    a, b, c = dumps[1], dumps[3], dumps[2]
+    for name, v in a.items():
+        assert v.dtype == np.float32 and np.isfinite(v).all(), name
+    assert a["loss"].shape == () and a["gradients"].shape == (1 << 22,)
+    assert float(np.abs(a["gradients"]).max()) > 0.0
+    assert rel_err(b["loss"], a["loss"]) < 1e-5 and rel_err(b["max_score"], a["max_score"]) < 1e-5
+    assert rel_err(b["gradients"], a["gradients"]) < 1e-3
+    # at the initial weights the loss sits near chance for any white-noise batch: batch 1 moves it by only ~1e-4
+    assert rel_err(c["loss"], a["loss"]) > 1e-5 and rel_err(c["gradients"], a["gradients"]) > 1e-2

@@ -502,6 +502,24 @@ def test_bench_reference_arm_prints_one_contract_line():
         ours = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1"], capture_output=True, text=True,
                               timeout=300, env=env)
         assert ours.returncode != 0 and "no CPU fallback" in (ours.stderr + ours.stdout)
+    # --dump-outputs is refused where there is no timed training step of ours to dump
+    refused = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs",
+                              "unused"], capture_output=True, text=True, timeout=120, env=env)
+    assert refused.returncode != 0 and "--dump-outputs" in refused.stderr and refused.stdout.strip() == ""
+
+
+def test_bench_dump_outputs_writes_float32_and_a_fixed_sample_of_long_arrays(tmp_path, monkeypatch):
+    import bench
+    monkeypatch.setattr(bench, "DUMP_SAMPLE", 1000)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"loss": torch.tensor(1.5, dtype=torch.float64),
+                                               "parameters": torch.arange(5000, dtype=torch.float64).view(50, 100)})
+    loss = np.load(tmp_path / "a" / "loss.npy")
+    assert loss.dtype == np.float32 and loss.shape == () and float(loss) == 1.5
+    a, b = np.load(tmp_path / "a" / "parameters.npy"), np.load(tmp_path / "b" / "parameters.npy")
+    assert a.dtype == np.float32 and a.shape == (1000,)
+    assert np.array_equal(a, b)                                   # the same entries on every run
+    assert bool((np.diff(a) > 0).all()) and a[0] >= 0 and a[-1] < 5000   # distinct entries, in index order
 
 
 def test_literal_loss_block_and_small_helpers():
