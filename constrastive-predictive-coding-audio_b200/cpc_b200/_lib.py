@@ -12,14 +12,14 @@ LIB_PATH = os.path.join(os.path.dirname(_HERE), "lib", "libcpc_b200.so")
 
 CQT_MAX_GROUPS = 16
 CQT_COMPLEX, CQT_LOGPOW, CQT_LOGPOW_PHASE = 0, 1, 2
-SCORE_LINEAR, SCORE_SOFTPLUS = 0, 1
+SCORE_LINEAR, SCORE_SOFTPLUS, SCORE_DIFFERENCE = 0, 1, 2
 CQT_FLAG_NO_TENSOR = 1
 CQT_FLAG_HALF_OPERANDS = 2
 CONV_FLAG_CUDA_CORE, CONV_FLAG_NO_TALL, CONV_FLAG_NO_SMALLK, CONV_FLAG_NO_FUSED_DGRAD = 1, 2, 4, 8
 CONV_FLAG_NO_MMA_SMALL_WGRAD = 16
 INFONCE_FLAG_NO_TENSOR = 1
 INFONCE_OUT_FLOATS = 4
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 
 class CqtParams(ctypes.Structure):

@@ -874,16 +874,27 @@ def _nce_key(tag, p):
     return "%s b%d k%d e%d %s" % (tag, p.batch, p.steps, p.enc, "all-steps" if p.all_steps else "per-step")
 
 
-def _nce_flops(p):
+def _nce_pairs_e(p):
     n = p.batch * p.steps
-    return 2.0 * n * n * p.enc if p.all_steps else 2.0 * p.steps * p.batch * p.batch * p.enc
+    return float(n * n * p.enc) if p.all_steps else float(p.steps * p.batch * p.batch * p.enc)
+
+
+def _nce_flops(p):
+    """Forward: the score tile, 2 operations per (pair, e) for a dot product, 3 for (p - z)^2 (subtract + fma)."""
+    return (3.0 if p.score_kind == _lib.SCORE_DIFFERENCE else 2.0) * _nce_pairs_e(p)
+
+
+def _nce_bwd_flops(p):
+    """Backward: the score tile recomputed, then the two tile products G.Z and G^T.P (2 operations each)."""
+    return _nce_flops(p) + 4.0 * _nce_pairs_e(p)
 
 
 def _nce_params(pred, targets, all_steps, kind, reg, precision):
     p = _lib.InfoNceParams()
     p.batch, p.steps, p.enc = pred.shape
     p.all_steps = int(bool(all_steps))
-    p.score_kind = {"linear": _lib.SCORE_LINEAR, "softplus": _lib.SCORE_SOFTPLUS}[kind]
+    p.score_kind = {"linear": _lib.SCORE_LINEAR, "softplus": _lib.SCORE_SOFTPLUS,
+                    "difference": _lib.SCORE_DIFFERENCE}[kind]
     p.regularization = float(reg)
     p.tgt_stride_b, p.tgt_stride_e, p.tgt_stride_k = targets.stride()
     p.precision = _PRECISION[precision]
@@ -927,7 +938,7 @@ class _InfoNceFunction(torch.autograd.Function):
         d_tgt = torch.empty(targets.shape, dtype=torch.float32, device=pred.device)
         ws = _workspace(lib.cpc_infonce_workspace_bytes(ctypes.byref(p), 1), pred.device)
         with torch.cuda.device(pred.device):
-            _call(_nce_key("cpc_infonce_bwd", p), 3.0 * _nce_flops(p), lib.cpc_infonce_bwd, _ptr(pred), _ptr(targets),
+            _call(_nce_key("cpc_infonce_bwd", p), _nce_bwd_flops(p), lib.cpc_infonce_bwd, _ptr(pred), _ptr(targets),
                   _ptr(lse), _ptr(g), _ptr(d_pred), _ptr(d_tgt), ctypes.byref(p), _ptr(ws),
                   ws.numel() if ws is not None else 0, _stream())
         return d_pred, d_tgt, None, None, None, None
@@ -936,7 +947,14 @@ class _InfoNceFunction(torch.autograd.Function):
 def infonce(pred, targets, all_steps, kind="linear", regularization=0.0, precision=None):
     """Fused InfoNCE.  pred (B,K,E), targets (B,E,K) (any strides).  Returns
     (loss, max_score, loss_without_regulariser, mean_score); only ``loss`` is differentiable.
-    Replaces contrastive_estimation_training.py:106-122,141,166."""
+    Replaces contrastive_estimation_training.py:106-122,141,166.
+
+    kind: "linear" (S = p.z), "softplus" (S = softplus(p.z)) or "difference" (S = 1 / |p - z|^2, the reference's
+    difference_score_function).  The difference kind always runs on the fp32 CUDA-core kernels with the squared
+    differences summed in fp32, so ``precision="bf16"`` gives bit-identical results to fp32 for it; a prediction equal
+    to a target gives S = +inf and a NaN loss.  The reference's literal block gives NaN too when that target is the
+    prediction's own, and +inf when it is another candidate's (its logsumexp keeps the +inf where the kernel's
+    max-shifted sum gives inf - inf); ``train()`` stops before the optimizer step on a NaN loss."""
     return _InfoNceFunction.apply(pred, targets, bool(all_steps), kind, float(regularization),
                                   precision or _default_precision)
 
@@ -944,7 +962,8 @@ def infonce(pred, targets, all_steps, kind="linear", regularization=0.0, precisi
 def infonce_validate(pred, targets, all_steps, kind="linear", precision=None):
     """Validation metrics of one batch (contrastive_estimation_training.py:224-247) without materialising the
     (B,K,B,K) score tensor: returns (per_step_losses (K), per_step_accuracy (K), mean_score ()).  The per-step
-    losses reproduce the reference's re-viewed ("scrambled") noise term in per-step mode (SURVEY.md Appendix B)."""
+    losses reproduce the reference's re-viewed ("scrambled") noise term in per-step mode (SURVEY.md Appendix B).
+    kind: "linear", "softplus" or "difference", as for ``infonce`` (the difference kind ignores ``precision``)."""
     _require_cuda(pred, targets)
     lib = _lib.load()
     if pred.dtype != torch.float32 or targets.dtype != torch.float32:

@@ -1,9 +1,11 @@
 """``ContrastiveEstimationTrainer`` with the fused InfoNCE kernels behind the reference's API.
 
 Constructor, ``train`` and ``validate`` signatures follow contrastive_estimation_training.py:36-269.  The
-three named score functions stay importable; when the trainer is given ``linear_score_function`` or
-``softplus_score_function`` the whole block ``score -> logsumexp -> loss -> regulariser -> max`` (:106-122,
-:141, :166) is ONE fused forward kernel family and one backward, and the (B,K,B,K) score tensor never exists.
+three named score functions stay importable; when the trainer is given ``linear_score_function``,
+``softplus_score_function`` or ``difference_score_function`` the whole block ``score -> logsumexp -> loss ->
+regulariser -> max`` (:106-122, :141, :166) is ONE fused forward kernel family and one backward, and the (B,K,B,K)
+score tensor never exists (nor, for the difference kind, the (B,K,E,B,K) tensor of differences).  Any other score
+function runs the literal block.
 
 Multi-GPU: one process per GPU.  Each rank trains on its contiguous slice of every batch, negatives stay on
 the rank, gradients are averaged by ``ddp.GradientBucketReducer`` while backward runs.
@@ -35,7 +37,8 @@ def difference_score_function(predicted_z, targets):
     return 1 / torch.sum(diff ** 2, dim=2)
 
 
-_FUSED_KINDS = {linear_score_function: "linear", softplus_score_function: "softplus"}
+_FUSED_KINDS = {linear_score_function: "linear", softplus_score_function: "softplus",
+                difference_score_function: "difference"}
 
 
 def reference_loss_from_scores(scores, batch_size, prediction_steps, all_steps, regularization):

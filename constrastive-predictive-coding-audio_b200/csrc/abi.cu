@@ -26,7 +26,7 @@ extern "C" const char* cpc_status_string(int status) {
         default: return "unknown status";
     }
 }
-extern "C" int cpc_abi_version(void) { return 6; }
+extern "C" int cpc_abi_version(void) { return 7; }
 extern "C" int cpc_runtime_check(void) { return cpc::check_device(); }
 extern "C" uint64_t cpc_launch_count(void) { return cpc::g_launches.load(); }
 extern "C" void cpc_launch_count_reset(void) { cpc::g_launches.store(0); }

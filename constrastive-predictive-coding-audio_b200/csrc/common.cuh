@@ -98,6 +98,35 @@ __device__ __forceinline__ void tile_gemm(const LA& la, const LB& lb, int row0, 
     }
 }
 
+// Same tiling, squared distances: acc[i][j] += sum_k (A(row, k) - B(col, k))^2.  The difference is formed before
+// squaring, so a near-coincident pair keeps its digits (|a|^2 + |b|^2 - 2 a.b would cancel them).  Out-of-range loads
+// are 0 on both sides and add nothing.
+template <class LA, class LB>
+__device__ __forceinline__ void tile_dist(const LA& la, const LB& lb, int row0, int col0, int k_begin, int k_end,
+                                          float (&acc)[4][4], TileSmem& sm) {
+    const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
+    for (int k0 = k_begin; k0 < k_end; k0 += TILE_K) {
+        tile_fill(la, sm.a, row0, k0);
+        tile_fill(lb, sm.b, col0, k0);
+        __syncthreads();
+#pragma unroll
+        for (int kk = 0; kk < TILE_K; ++kk) {
+            const float4 a = *reinterpret_cast<const float4*>(&sm.a[kk][tx * 4]);
+            const float4 b = *reinterpret_cast<const float4*>(&sm.b[kk][ty * 4]);
+            const float av[4] = {a.x, a.y, a.z, a.w};
+            const float bv[4] = {b.x, b.y, b.z, b.w};
+#pragma unroll
+            for (int i = 0; i < 4; ++i)
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    const float d = av[i] - bv[j];
+                    acc[i][j] = fmaf(d, d, acc[i][j]);
+                }
+        }
+        __syncthreads();
+    }
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

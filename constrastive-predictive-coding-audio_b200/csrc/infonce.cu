@@ -5,6 +5,8 @@
 // Notation (SURVEY.md Appendix B): P = pred (B,K,E), Z = targets (B,E,K) strided view.
 //   all-steps mode : one problem, rows r=(d,k), columns c=(t,k');  S[r,c] = phi(P[r,:] . Z[t,:,k'])
 //   per-step mode  : K problems,  rows d,     columns t;           S_k[d,t] = phi(P[d,k,:] . Z[t,:,k])
+// phi is the identity (linear) or softplus; the difference kind scores S = 1 / D with D = |P[r,:] - Z[c,:]|^2, summed
+// as squared differences in fp32 (tile_dist), never as |p|^2 + |z|^2 - 2 p.z.
 // loss = mean_c (lse_r S[:,c] - S[c,c]) + lambda * mean((mean_k S)^2).  The reference's per-step
 // ".view" scramble is a bijection under the mean, so the training loss equals this clean form.
 //
@@ -44,7 +46,8 @@ static int nce_validate(const cpc_infonce_params* p) {
     if (p->batch <= 0 || p->steps <= 0 || p->enc <= 0) return CPC_ERR_BAD_SHAPE;
     if (p->steps > TILE) return CPC_ERR_UNSUPPORTED;
     if ((int64_t)p->batch * p->steps > (1 << 30)) return CPC_ERR_BAD_SHAPE;
-    if (p->score_kind != CPC_SCORE_LINEAR && p->score_kind != CPC_SCORE_SOFTPLUS) return CPC_ERR_BAD_SHAPE;
+    if (p->score_kind != CPC_SCORE_LINEAR && p->score_kind != CPC_SCORE_SOFTPLUS && p->score_kind != CPC_SCORE_DIFFERENCE)
+        return CPC_ERR_BAD_SHAPE;
     return CPC_OK;
 }
 
@@ -102,6 +105,27 @@ __device__ __forceinline__ float softplus_f(float u) {   // torch F.softplus(bet
 }
 __device__ __forceinline__ float sigmoid_f(float u) { return 1.f / (1.f + expf(-u)); }
 
+// The kernels below are instantiated twice: kDiff = false for the dot-product kinds (linear, softplus: g.kind picks
+// phi at run time), kDiff = true for the difference kind, so that neither pays registers for the other's code.
+// One problem's 64x64 tile of score arguments: the dot product u, or the squared distance D.
+template <bool kDiff, class LA, class LB>
+__device__ __forceinline__ void score_tile(const NceGeom& g, const LA& la, const LB& lb, int row0, int col0,
+                                           float (&acc)[4][4], TileSmem& sm) {
+    if (kDiff) tile_dist(la, lb, row0, col0, 0, g.E, acc, sm);
+    else tile_gemm(la, lb, row0, col0, 0, g.E, acc, sm);
+}
+// Score from the tile value.  D = 0 gives S = +inf, as the reference's 1 / sum(diff ** 2) does: no epsilon.  The loss
+// is then NaN (expf(inf - inf) in the column statistics); the reference's is NaN when the coinciding target is the
+// prediction's own and +inf when it is another candidate's (torch.logsumexp keeps the +inf).
+template <bool kDiff>
+__device__ __forceinline__ float score_of(int kind, float a) {
+    // hardware reciprocal: the IEEE division's slow-path call made the backward spill; 1/0 = +inf.  Within 2 ulp of
+    // 1/D for D in [2^-126, 2^126]; outside (a prediction within ~1e-19 of a target, or |p - z| > 1e19) it flushes to
+    // +inf / 0 where IEEE 1/D would still be finite / denormal.
+    if (kDiff) return __fdividef(1.f, a);
+    return kind == CPC_SCORE_SOFTPLUS ? softplus_f(a) : a;
+}
+
 __device__ __forceinline__ PRows make_p(const float* p, const NceGeom& g, int prob) {
     return g.all ? PRows{p, g.R, g.E, 0, g.E} : PRows{p, g.R, g.E, (long long)prob * g.E, (long long)g.K * g.E};
 }
@@ -146,6 +170,7 @@ __device__ __forceinline__ float block_max(float v, float* red) {
 // which left the raw-wave configuration (B = 8 ... 64, K = 12: ONE tile) on a single SM for 0.6 - 0.9 ms.  Its
 // regulariser couples the problems (mean over k of S_k[d, t]): the CTAs add their scores into rsum (R x C, zeroed by the
 // caller) and nce_final_kernel squares the means.
+template <bool kDiff>
 __global__ void __launch_bounds__(TILE_THREADS) nce_fwd_kernel(const float* __restrict__ P, const float* __restrict__ Z,
                                                               NceGeom g, float* __restrict__ part_m,
                                                               float* __restrict__ part_s, float* __restrict__ diag,
@@ -162,7 +187,7 @@ __global__ void __launch_bounds__(TILE_THREADS) nce_fwd_kernel(const float* __re
     {
         const int prob = blockIdx.z;
         float acc[4][4] = {};
-        tile_gemm(make_p(P, g, prob), make_z(Z, g, prob), row0, col0, 0, g.E, acc, sm);
+        score_tile<kDiff>(g, make_p(P, g, prob), make_z(Z, g, prob), row0, col0, acc, sm);
         float s[4][4];
         bool ok[4][4];
 #pragma unroll
@@ -171,7 +196,7 @@ __global__ void __launch_bounds__(TILE_THREADS) nce_fwd_kernel(const float* __re
             for (int j = 0; j < 4; ++j) {
                 const int lr = tx * 4 + i, r = row0 + lr, c = col0 + ty * 4 + j;
                 ok[i][j] = lr < g.tmr && r < g.R && c < g.C;
-                const float v = g.kind == CPC_SCORE_SOFTPLUS ? softplus_f(acc[i][j]) : acc[i][j];
+                const float v = score_of<kDiff>(g.kind, acc[i][j]);
                 s[i][j] = ok[i][j] ? v : -INFINITY;
                 if (ok[i][j]) {
                     tmax = fmaxf(tmax, v);
@@ -337,6 +362,7 @@ __global__ void __launch_bounds__(256) nce_validate_final_kernel(const float* __
 
 // ---- backward -----------------------------------------------------------------------------------
 // Per-step regulariser, pass 1: rsum[d, t] += S_k[d, t] for every step k (grid (col tiles, row tiles, K); rsum zeroed).
+template <bool kDiff>
 __global__ void __launch_bounds__(TILE_THREADS) nce_rsum_kernel(const float* __restrict__ P, const float* __restrict__ Z,
                                                                NceGeom g, float* __restrict__ rsum) {
     __shared__ TileSmem sm;
@@ -344,20 +370,25 @@ __global__ void __launch_bounds__(TILE_THREADS) nce_rsum_kernel(const float* __r
     const int col0 = blockIdx.x * TILE, row0 = blockIdx.y * g.tmr;
     const int prob = blockIdx.z;
     float acc[4][4] = {};
-    tile_gemm(make_p(P, g, prob), make_z(Z, g, prob), row0, col0, 0, g.E, acc, sm);
+    score_tile<kDiff>(g, make_p(P, g, prob), make_z(Z, g, prob), row0, col0, acc, sm);
 #pragma unroll
     for (int i = 0; i < 4; ++i)
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
             const int lr = tx * 4 + i, r = row0 + lr, c = col0 + ty * 4 + j;
             if (lr < g.tmr && r < g.R && c < g.C)
-                atomicAdd(rsum + (size_t)r * g.C + c, g.kind == CPC_SCORE_SOFTPLUS ? softplus_f(acc[i][j]) : acc[i][j]);
+                atomicAdd(rsum + (size_t)r * g.C + c, score_of<kDiff>(g.kind, acc[i][j]));
         }
 }
 
 // grid (col tiles, row tiles, problems x esplit): a CTA recomputes the score tile of ONE problem and produces the
 // gradient columns e = (es + n * esplit) * 64 ... of it (small problems -- one or a few tiles -- are spread over the SMs by
 // the problem and by the slice of E; they used to run their K problems and 8 slices one after the other on one SM).
+// Difference kind: with H = G * S^2 (dS/dD = -S^2) the tile holds Gs = 2H, and
+//   dP[r,:] = -2 sum_c H[r,c] (P[r,:] - Z[c,:]) = (Gs Zc)[r,:] - h_r P[r,:],   h_r  = sum_c Gs[r,c]
+//   dZc[c,:] = 2 sum_r H[r,c] (P[r,:] - Z[c,:]) = (Gs^T P)[c,:] - h'_c Z[c,:],  h'_c = sum_r Gs[r,c]
+// so the two tile products stay as they are and each CTA adds its tile's share of the rank-1 terms.
+template <bool kDiff>
 __global__ void __launch_bounds__(TILE_THREADS) nce_bwd_kernel(const float* __restrict__ P, const float* __restrict__ Z,
                                                               const float* __restrict__ lse,
                                                               const float* __restrict__ grad_loss, NceGeom g,
@@ -366,6 +397,7 @@ __global__ void __launch_bounds__(TILE_THREADS) nce_bwd_kernel(const float* __re
     __shared__ TileSmem sm;
     __shared__ float Gs[TILE][TILE + 1];
     __shared__ float Sbar[TILE][TILE];         // all-steps regulariser: (group, column); groups = tmr/K <= 64
+    __shared__ float hrow[TILE], hcol[TILE];   // difference kind: row / column sums of Gs over this tile
     const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
     const int col0 = blockIdx.x * TILE, row0 = blockIdx.y * g.tmr;
     const float gl = __ldg(grad_loss);
@@ -388,12 +420,12 @@ __global__ void __launch_bounds__(TILE_THREADS) nce_bwd_kernel(const float* __re
         const PRows pr = make_p(P, g, prob);
         const ZRows zr = make_z(Z, g, prob);
         float acc[4][4] = {};
-        tile_gemm(pr, zr, row0, col0, 0, g.E, acc, sm);
+        score_tile<kDiff>(g, pr, zr, row0, col0, acc, sm);
         float s[4][4];
 #pragma unroll
         for (int i = 0; i < 4; ++i)
 #pragma unroll
-            for (int j = 0; j < 4; ++j) s[i][j] = g.kind == CPC_SCORE_SOFTPLUS ? softplus_f(acc[i][j]) : acc[i][j];
+            for (int j = 0; j < 4; ++j) s[i][j] = score_of<kDiff>(g.kind, acc[i][j]);
         if (g.all && g.lambda != 0.f) {
 #pragma unroll
             for (int i = 0; i < 4; ++i)
@@ -428,11 +460,25 @@ __global__ void __launch_bounds__(TILE_THREADS) nce_bwd_kernel(const float* __re
                 if (ok) {
                     const float l = __ldg(lse + (size_t)prob * g.C + c);
                     gv = w_ce * (expf(s[i][j] - l) - (r == c ? 1.f : 0.f)) + w_reg * sbar[i][j];
-                    if (g.kind == CPC_SCORE_SOFTPLUS) gv *= sigmoid_f(acc[i][j]);
+                    if (kDiff) gv *= 2.f * s[i][j] * s[i][j];
+                    else if (g.kind == CPC_SCORE_SOFTPLUS) gv *= sigmoid_f(acc[i][j]);
                 }
                 Gs[lr][ty * 4 + j] = gv;
             }
         __syncthreads();
+        if (kDiff) {                                  // entries outside the problem are 0 in Gs
+            if (threadIdx.x < TILE) {
+                float a = 0.f;
+                for (int cc = 0; cc < TILE; ++cc) a += Gs[threadIdx.x][cc];
+                hrow[threadIdx.x] = a;
+            } else if (threadIdx.x < 2 * TILE) {
+                const int cc = threadIdx.x - TILE;
+                float a = 0.f;
+                for (int rr = 0; rr < TILE; ++rr) a += Gs[rr][cc];
+                hcol[cc] = a;
+            }
+            __syncthreads();
+        }
         for (int e0 = es * TILE; e0 < g.E; e0 += esplit * TILE) {
             {   // dP[r, e] += sum_c G[r,c] Zc[c,e]
                 float a2[4][4] = {};
@@ -444,7 +490,10 @@ __global__ void __launch_bounds__(TILE_THREADS) nce_bwd_kernel(const float* __re
 #pragma unroll
                     for (int j = 0; j < 4; ++j) {
                         const int e = e0 + ty * 4 + j;
-                        if (e < g.E) atomicAdd(dP + pr.base + (long long)r * pr.stride + e, a2[i][j]);
+                        if (e >= g.E) continue;
+                        float v = a2[i][j];
+                        if (kDiff) v -= hrow[lr] * pr.load(r, e);
+                        atomicAdd(dP + pr.base + (long long)r * pr.stride + e, v);
                     }
                 }
             }
@@ -460,13 +509,20 @@ __global__ void __launch_bounds__(TILE_THREADS) nce_bwd_kernel(const float* __re
 #pragma unroll
                     for (int j = 0; j < 4; ++j) {
                         const int e = e0 + ty * 4 + j;
-                        if (e < g.E) atomicAdd(dZ + ((size_t)t * g.E + e) * g.K + kk, a3[i][j]);
+                        if (e >= g.E) continue;
+                        float v = a3[i][j];
+                        if (kDiff) v -= hcol[tx * 4 + i] * zr.load(c, e);
+                        atomicAdd(dZ + ((size_t)t * g.E + e) * g.K + kk, v);
                     }
                 }
             }
         }
         __syncthreads();
     }
+}
+
+static decltype(&nce_fwd_kernel<false>) nce_fwd_launcher(const NceGeom& g) {
+    return g.kind == CPC_SCORE_DIFFERENCE ? nce_fwd_kernel<true> : nce_fwd_kernel<false>;
 }
 
 struct NceWs {
@@ -534,8 +590,8 @@ extern "C" int cpc_infonce_fwd(const float* pred, const float* targets, float* o
     const size_t n_rsum = nce_rsum_floats(g);
     if (n_rsum && cudaMemsetAsync(w.rsum, 0, sizeof(float) * n_rsum, s) != cudaSuccess) return CPC_ERR_CUDA;
     dim3 grid(ceil_div(g.C, TILE), g.nrowtiles, g.nprob);
-    nce_fwd_kernel<<<grid, TILE_THREADS, 0, s>>>(pred, targets, g, w.part_m, w.part_s, w.diag, w.cta, nullptr, nullptr,
-                                                 n_rsum ? w.rsum : nullptr);
+    nce_fwd_launcher(g)<<<grid, TILE_THREADS, 0, s>>>(pred, targets, g, w.part_m, w.part_s, w.diag, w.cta, nullptr,
+                                                      nullptr, n_rsum ? w.rsum : nullptr);
     CPC_LAUNCH_CHECK();
     nce_combine_kernel<<<w.nblk, 256, 0, s>>>(w.part_m, w.part_s, w.diag, lse, w.blk, g.ncols, g.nrowtiles);
     CPC_LAUNCH_CHECK();
@@ -566,13 +622,15 @@ extern "C" int cpc_infonce_bwd(const float* pred, const float* targets, const fl
         if (!workspace || workspace_bytes < sizeof(float) * n_rsum) return CPC_ERR_WORKSPACE;
         rsum = reinterpret_cast<float*>(workspace);
         if (cudaMemsetAsync(rsum, 0, sizeof(float) * n_rsum, s) != cudaSuccess) return CPC_ERR_CUDA;
-        nce_rsum_kernel<<<dim3(ceil_div(g.C, TILE), g.nrowtiles, g.nprob), TILE_THREADS, 0, s>>>(pred, targets, g, rsum);
+        auto rsum_kernel = g.kind == CPC_SCORE_DIFFERENCE ? nce_rsum_kernel<true> : nce_rsum_kernel<false>;
+        rsum_kernel<<<dim3(ceil_div(g.C, TILE), g.nrowtiles, g.nprob), TILE_THREADS, 0, s>>>(pred, targets, g, rsum);
         CPC_LAUNCH_CHECK();
         count_launch();
     }
     const int esplit = nce_esplit(g);
     dim3 grid(ceil_div(g.C, TILE), g.nrowtiles, g.nprob * esplit);
-    nce_bwd_kernel<<<grid, TILE_THREADS, 0, s>>>(pred, targets, lse, grad_loss, g, d_pred, d_targets, rsum, esplit);
+    auto bwd_kernel = g.kind == CPC_SCORE_DIFFERENCE ? nce_bwd_kernel<true> : nce_bwd_kernel<false>;
+    bwd_kernel<<<grid, TILE_THREADS, 0, s>>>(pred, targets, lse, grad_loss, g, d_pred, d_targets, rsum, esplit);
     CPC_LAUNCH_CHECK();
     count_launch();
     return CPC_OK;
@@ -600,7 +658,8 @@ extern "C" int cpc_infonce_validate(const float* pred, const float* targets, flo
     int* rowp_i = reinterpret_cast<int*>(base + align_up(sizeof(float) * rows, 256));
     cudaStream_t s = (cudaStream_t)stream;
     dim3 grid(ncoltiles, g.nrowtiles, g.nprob);
-    nce_fwd_kernel<<<grid, TILE_THREADS, 0, s>>>(pred, targets, g, w.part_m, w.part_s, w.diag, w.cta, rowp_m, rowp_i, nullptr);
+    nce_fwd_launcher(g)<<<grid, TILE_THREADS, 0, s>>>(pred, targets, g, w.part_m, w.part_s, w.diag, w.cta, rowp_m, rowp_i,
+                                                      nullptr);
     CPC_LAUNCH_CHECK();
     nce_combine_kernel<<<w.nblk, 256, 0, s>>>(w.part_m, w.part_s, w.diag, lse, w.blk, g.ncols, g.nrowtiles);
     CPC_LAUNCH_CHECK();

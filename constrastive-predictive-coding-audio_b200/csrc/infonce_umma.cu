@@ -561,6 +561,9 @@ __global__ void __launch_bounds__(NU_THREADS, 1) nce_umma_bwd_kernel(const __gri
 // ---- host side ----------------------------------------------------------------------------------------------
 // which: 0 forward, 1 backward
 bool nce_umma_eligible(const cpc_infonce_params* p, int which) {
+    // the kernels below compute dot products only (any other kind would run as linear), and a distance from them would
+    // be |p|^2 + |z|^2 - 2 p.z, which cancels for the near pairs the difference kind is about
+    if (p->score_kind == CPC_SCORE_DIFFERENCE) return false;
     if (p->enc % 64 != 0 || p->enc < 64 || p->enc > 4096) return false;
     const long bp = p->all_steps ? (long)p->batch * p->steps : p->batch;
     if (bp < 128 || bp > (1 << 24)) return false;                          // tiny problems are latency-bound either way

@@ -271,7 +271,14 @@ int cpc_maxpool_bwd_accumulate(const float* x, const float* dy, float* dx, const
  *    pred (B, K, E) contiguous fp32; targets is the *strided view* z[:, :, -K:] of the encoder output
  *    (audio_model.py:197): element (t, e, k) at targets[t*tgt_stride_b + e*tgt_stride_e + k*tgt_stride_k].
  * ---------------------------------------------------------------------------------------------- */
-typedef enum cpc_score_kind { CPC_SCORE_LINEAR = 0, CPC_SCORE_SOFTPLUS = 1 } cpc_score_kind;
+typedef enum cpc_score_kind {
+    CPC_SCORE_LINEAR = 0,
+    CPC_SCORE_SOFTPLUS = 1,
+    /* difference_score_function (contrastive_estimation_training.py): S = 1 / sum_e (P[r,e] - Z[c,e])^2.  Always on
+     * the fp32 CUDA-core kernels (also with precision = bf16), with the squared differences accumulated in fp32, never
+     * expanded as |p|^2 + |z|^2 - 2 p.z; a prediction equal to a target gives S = +inf and a NaN loss. */
+    CPC_SCORE_DIFFERENCE = 2
+} cpc_score_kind;
 
 typedef struct cpc_infonce_params {
     int32_t batch;          /* B */
