@@ -62,6 +62,10 @@ class InfoNceParams(ctypes.Structure):
                 ("precision", ctypes.c_int32), ("flags", ctypes.c_int32)]
 
 
+class InfoNceShard(ctypes.Structure):
+    _fields_ = [("pred_batch", ctypes.c_int32), ("target_offset", ctypes.c_int32)]
+
+
 class AdamParams(ctypes.Structure):
     _fields_ = [("lr", ctypes.c_double), ("beta1", ctypes.c_double), ("beta2", ctypes.c_double), ("eps", ctypes.c_double),
                 ("weight_decay", ctypes.c_double), ("grad_scale", ctypes.c_float), ("maximize", ctypes.c_int32)]
@@ -111,6 +115,12 @@ SIGNATURES = {
     "cpc_infonce_fwd": (ctypes.c_int, [_P, _P, _P, _P, ctypes.POINTER(InfoNceParams), _P, ctypes.c_size_t, _P]),
     "cpc_infonce_bwd": (ctypes.c_int, [_P, _P, _P, _P, _P, _P, ctypes.POINTER(InfoNceParams), _P, ctypes.c_size_t, _P]),
     "cpc_infonce_validate": (ctypes.c_int, [_P, _P, _P, ctypes.POINTER(InfoNceParams), _P, ctypes.c_size_t, _P]),
+    "cpc_infonce_workspace_bytes_ex": (ctypes.c_size_t, [ctypes.POINTER(InfoNceParams), ctypes.POINTER(InfoNceShard),
+                                                         ctypes.c_int]),
+    "cpc_infonce_fwd_ex": (ctypes.c_int, [_P, _P, _P, _P, ctypes.POINTER(InfoNceParams), ctypes.POINTER(InfoNceShard), _P,
+                                          ctypes.c_size_t, _P]),
+    "cpc_infonce_bwd_ex": (ctypes.c_int, [_P, _P, _P, _P, _P, _P, ctypes.POINTER(InfoNceParams),
+                                          ctypes.POINTER(InfoNceShard), _P, ctypes.c_size_t, _P]),
     "cpc_adam_step": (ctypes.c_int, [ctypes.c_int32, _P, _P, _P, _P, _P, _P, ctypes.POINTER(AdamParams), _P]),
 }
 

@@ -2,8 +2,17 @@
 issued from autograd hooks while backward is still running (SURVEY.md 8e).
 
 The reference uses single-process ``nn.DataParallel`` (setup_functions.py:112-115).  Here every rank owns a
-contiguous slice of each batch -- the same dim-0 chunking ``DataParallel.scatter`` applies -- and negatives
-stay on the rank (north star), so the forward pass needs no collective at all.
+contiguous slice of each batch -- the same dim-0 chunking ``DataParallel.scatter`` applies.
+
+Negatives.  By default they stay on the rank (north star): each rank scores its shard against its own predictions and
+the forward pass needs no collective at all; the loss is the mean of W shard losses, not the reference's.  Opt-in,
+``ContrastiveEstimationTrainer(global_negatives=True)`` reproduces what DataParallel computes on the outputs it gathers
+onto one GPU: every target is ranked against the predictions of the whole global batch.  Each rank all-gathers the
+predictions (``gather_predictions``), scores its own targets against them (a rectangular ``ops.infonce`` call) and
+back-propagates its shard loss L_r; the backward of the gather reduce-scatters the prediction gradients with SUM.
+Since mean_r L_r is the global loss, that sum is W times the global gradient of this rank's predictions, and the
+usual averaging of the parameter gradients over W leaves exactly the global gradient.  BatchNorm statistics stay per
+rank, as in DataParallel's replicas.
 """
 import os
 
@@ -63,6 +72,50 @@ class ShardedBatchSampler(torch.utils.data.Sampler):
 
     def __len__(self):
         return len(self.batch_sampler)
+
+
+class _GatherPredictions(torch.autograd.Function):
+    """Forward: all-gather of the ranks' (b, ...) tensors into (W*b, ...) in rank order.  Backward: reduce-scatter (SUM)
+    of the gathered gradient, each rank keeping its own rows.  Both are plain synchronous collectives, ordered with the
+    current stream, so they can be captured in a CUDA graph (GraphedTrainStep)."""
+
+    @staticmethod
+    def forward(ctx, x, group):
+        ctx.group = group
+        world = dist.get_world_size(group)
+        x = x.contiguous()
+        out = x.new_empty((world * x.shape[0],) + tuple(x.shape[1:]))
+        dist.all_gather_into_tensor(out, x, group=group)
+        return out
+
+    @staticmethod
+    def backward(ctx, grad):
+        world = dist.get_world_size(ctx.group)
+        grad = grad.contiguous()
+        out = grad.new_empty((grad.shape[0] // world,) + tuple(grad.shape[1:]))
+        # NCCL calls on one communicator must be issued in the same order on every rank.  This one is issued when
+        # autograd reaches the gather node, right after the InfoNCE node's backward: the gather is the newest node on
+        # every path from the predictions to the loss, so no parameter gradient is final yet and no gradient-bucket
+        # all-reduce hook has fired.  Keep the gather directly in front of the InfoNCE call to keep it so.
+        dist.reduce_scatter_tensor(out, grad, op=dist.ReduceOp.SUM, group=ctx.group)
+        return out, None
+
+
+def gather_predictions(x, group=None):
+    """All ranks' ``x`` concatenated along dim 0 in rank order, differentiable: the gradient that reaches each rank's
+    ``x`` is the SUM over ranks of the gradients of the gathered tensor at its rows."""
+    return _GatherPredictions.apply(x, group)
+
+
+def combine_shard_losses(loss_r, max_r, group=None):
+    """(L_r, max_r) of each rank -> (loss, max) with the value of mean_r L_r and of max_r max_r on every rank, from one
+    all-gather of a 2-vector.  The loss keeps the gradient of L_r: ``L_r + (mean - L_r).detach()``."""
+    world = dist.get_world_size(group)
+    local = torch.stack([loss_r.detach().reshape(()), max_r.detach().reshape(())]).to(loss_r.dtype)
+    both = local.new_empty(2 * world)
+    dist.all_gather_into_tensor(both, local, group=group)
+    both = both.view(world, 2)
+    return loss_r + (both[:, 0].mean() - loss_r).detach(), both[:, 1].max()
 
 
 def broadcast_parameters(module, src=0):

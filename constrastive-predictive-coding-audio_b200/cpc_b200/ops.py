@@ -870,28 +870,43 @@ def max_pool2d(x, kernel, ceil_mode=False):
 # InfoNCE
 # --------------------------------------------------------------------------------------------------
 
-def _nce_key(tag, p):
-    return "%s b%d k%d e%d %s" % (tag, p.batch, p.steps, p.enc, "all-steps" if p.all_steps else "per-step")
+def _nce_key(tag, p, shard=None):
+    rect = "" if shard is None else " x%d" % shard.pred_batch
+    return "%s b%d%s k%d e%d %s" % (tag, p.batch, rect, p.steps, p.enc, "all-steps" if p.all_steps else "per-step")
 
 
-def _nce_pairs_e(p):
-    n = p.batch * p.steps
-    return float(n * n * p.enc) if p.all_steps else float(p.steps * p.batch * p.batch * p.enc)
+def _nce_pairs_e(p, shard=None):
+    """(prediction, target) pairs scored, times E: the square problem, or the rectangle of a shard call."""
+    rows = p.batch if shard is None else shard.pred_batch
+    if p.all_steps:
+        return float(rows * p.steps * p.batch * p.steps * p.enc)
+    return float(p.steps * rows * p.batch * p.enc)
 
 
-def _nce_flops(p):
+def _nce_flops(p, shard=None):
     """Forward: the score tile, 2 operations per (pair, e) for a dot product, 3 for (p - z)^2 (subtract + fma)."""
-    return (3.0 if p.score_kind == _lib.SCORE_DIFFERENCE else 2.0) * _nce_pairs_e(p)
+    return (3.0 if p.score_kind == _lib.SCORE_DIFFERENCE else 2.0) * _nce_pairs_e(p, shard)
 
 
-def _nce_bwd_flops(p):
+def _nce_bwd_flops(p, shard=None):
     """Backward: the score tile recomputed, then the two tile products G.Z and G^T.P (2 operations each)."""
-    return _nce_flops(p) + 4.0 * _nce_pairs_e(p)
+    return _nce_flops(p, shard) + 4.0 * _nce_pairs_e(p, shard)
+
+
+def _nce_shard(pred, targets, target_offset):
+    """None for the square problem (pred and targets hold the same items); otherwise the rectangle of a shard call:
+    targets' items scored against all pred.shape[0] predictions, positive of target t at prediction target_offset + t."""
+    if pred.shape[0] == targets.shape[0] and target_offset == 0:
+        return None
+    sh = _lib.InfoNceShard()
+    sh.pred_batch, sh.target_offset = pred.shape[0], int(target_offset)
+    return sh
 
 
 def _nce_params(pred, targets, all_steps, kind, reg, precision):
     p = _lib.InfoNceParams()
-    p.batch, p.steps, p.enc = pred.shape
+    p.steps, p.enc = pred.shape[1:]
+    p.batch = targets.shape[0]
     p.all_steps = int(bool(all_steps))
     p.score_kind = {"linear": _lib.SCORE_LINEAR, "softplus": _lib.SCORE_SOFTPLUS,
                     "difference": _lib.SCORE_DIFFERENCE}[kind]
@@ -904,23 +919,31 @@ def _nce_params(pred, targets, all_steps, kind, reg, precision):
 
 class _InfoNceFunction(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, pred, targets, all_steps, kind, reg, precision):
+    def forward(ctx, pred, targets, all_steps, kind, reg, precision, target_offset):
         _require_cuda(pred, targets)
         lib = _lib.load()
         if pred.dtype != torch.float32 or targets.dtype != torch.float32:
             raise _lib.CpcError("infonce expects fp32 tensors")
-        b, k, e = pred.shape
+        _, k, e = pred.shape
+        b = targets.shape[0]
         if tuple(targets.shape) != (b, e, k):
             raise ValueError("targets must be (B, E, K) = %s, got %s" % ((b, e, k), tuple(targets.shape)))
         pred = pred.contiguous()
         p = _nce_params(pred, targets, all_steps, kind, reg, precision)
+        sh = _nce_shard(pred, targets, target_offset)
         out = torch.empty(_lib.INFONCE_OUT_FLOATS, dtype=torch.float32, device=pred.device)
         lse = torch.empty(b * k, dtype=torch.float32, device=pred.device)
-        ws = _workspace(lib.cpc_infonce_workspace_bytes(ctypes.byref(p), 0), pred.device)
         with torch.cuda.device(pred.device):
-            _call(_nce_key("cpc_infonce_fwd", p), _nce_flops(p), lib.cpc_infonce_fwd, _ptr(pred), _ptr(targets),
-                  _ptr(out), _ptr(lse), ctypes.byref(p), _ptr(ws), ws.numel() if ws is not None else 0, _stream())
-        ctx.args = (all_steps, kind, reg, precision)
+            if sh is None:
+                ws = _workspace(lib.cpc_infonce_workspace_bytes(ctypes.byref(p), 0), pred.device)
+                _call(_nce_key("cpc_infonce_fwd", p), _nce_flops(p), lib.cpc_infonce_fwd, _ptr(pred), _ptr(targets),
+                      _ptr(out), _ptr(lse), ctypes.byref(p), _ptr(ws), ws.numel() if ws is not None else 0, _stream())
+            else:
+                ws = _workspace(lib.cpc_infonce_workspace_bytes_ex(ctypes.byref(p), ctypes.byref(sh), 0), pred.device)
+                _call(_nce_key("cpc_infonce_fwd_ex", p, sh), _nce_flops(p, sh), lib.cpc_infonce_fwd_ex, _ptr(pred),
+                      _ptr(targets), _ptr(out), _ptr(lse), ctypes.byref(p), ctypes.byref(sh), _ptr(ws),
+                      ws.numel() if ws is not None else 0, _stream())
+        ctx.args = (all_steps, kind, reg, precision, target_offset)
         ctx.save_for_backward(pred, targets, lse)
         loss, max_score, loss_noreg, mean_score = out[0], out[1], out[2], out[3]
         ctx.mark_non_differentiable(max_score, loss_noreg, mean_score)
@@ -931,23 +954,36 @@ class _InfoNceFunction(torch.autograd.Function):
     def backward(ctx, g_loss, _g1, _g2, _g3):
         pred, targets, lse = ctx.saved_tensors
         lib = _lib.load()
-        all_steps, kind, reg, precision = ctx.args
+        all_steps, kind, reg, precision, target_offset = ctx.args
         p = _nce_params(pred, targets, all_steps, kind, reg, precision)
+        sh = _nce_shard(pred, targets, target_offset)
         g = g_loss.reshape(1).to(torch.float32).contiguous()
         d_pred = torch.empty_like(pred)
         d_tgt = torch.empty(targets.shape, dtype=torch.float32, device=pred.device)
-        ws = _workspace(lib.cpc_infonce_workspace_bytes(ctypes.byref(p), 1), pred.device)
         with torch.cuda.device(pred.device):
-            _call(_nce_key("cpc_infonce_bwd", p), _nce_bwd_flops(p), lib.cpc_infonce_bwd, _ptr(pred), _ptr(targets),
-                  _ptr(lse), _ptr(g), _ptr(d_pred), _ptr(d_tgt), ctypes.byref(p), _ptr(ws),
-                  ws.numel() if ws is not None else 0, _stream())
-        return d_pred, d_tgt, None, None, None, None
+            if sh is None:
+                ws = _workspace(lib.cpc_infonce_workspace_bytes(ctypes.byref(p), 1), pred.device)
+                _call(_nce_key("cpc_infonce_bwd", p), _nce_bwd_flops(p), lib.cpc_infonce_bwd, _ptr(pred), _ptr(targets),
+                      _ptr(lse), _ptr(g), _ptr(d_pred), _ptr(d_tgt), ctypes.byref(p), _ptr(ws),
+                      ws.numel() if ws is not None else 0, _stream())
+            else:
+                ws = _workspace(lib.cpc_infonce_workspace_bytes_ex(ctypes.byref(p), ctypes.byref(sh), 1), pred.device)
+                _call(_nce_key("cpc_infonce_bwd_ex", p, sh), _nce_bwd_flops(p, sh), lib.cpc_infonce_bwd_ex, _ptr(pred),
+                      _ptr(targets), _ptr(lse), _ptr(g), _ptr(d_pred), _ptr(d_tgt), ctypes.byref(p), ctypes.byref(sh),
+                      _ptr(ws), ws.numel() if ws is not None else 0, _stream())
+        return d_pred, d_tgt, None, None, None, None, None
 
 
-def infonce(pred, targets, all_steps, kind="linear", regularization=0.0, precision=None):
+def infonce(pred, targets, all_steps, kind="linear", regularization=0.0, precision=None, target_offset=0):
     """Fused InfoNCE.  pred (B,K,E), targets (B,E,K) (any strides).  Returns
     (loss, max_score, loss_without_regulariser, mean_score); only ``loss`` is differentiable.
     Replaces contrastive_estimation_training.py:106-122,141,166.
+
+    Shard call: pred (B_all,K,E) with B_all > B (the gathered predictions of every data-parallel rank), targets this
+    rank's (B,E,K), the positive of target t at prediction ``target_offset + t``.  The loss is the reference's block on
+    that column block of the global score tensor (logsumexp over all B_all candidates, mean over this rank's columns,
+    regulariser, max and mean score over the block): for W equal shards at offsets r * B, the mean of the W losses is
+    the global loss and their pred gradients sum to W times the global one (``ddp.gather_predictions``).
 
     kind: "linear" (S = p.z), "softplus" (S = softplus(p.z)) or "difference" (S = 1 / |p - z|^2, the reference's
     difference_score_function).  The difference kind always runs on the fp32 CUDA-core kernels with the squared
@@ -956,7 +992,7 @@ def infonce(pred, targets, all_steps, kind="linear", regularization=0.0, precisi
     prediction's own, and +inf when it is another candidate's (its logsumexp keeps the +inf where the kernel's
     max-shifted sum gives inf - inf); ``train()`` stops before the optimizer step on a NaN loss."""
     return _InfoNceFunction.apply(pred, targets, bool(all_steps), kind, float(regularization),
-                                  precision or _default_precision)
+                                  precision or _default_precision, int(target_offset))
 
 
 def infonce_validate(pred, targets, all_steps, kind="linear", precision=None):

@@ -7,8 +7,10 @@ regulariser -> max`` (:106-122, :141, :166) is ONE fused forward kernel family a
 score tensor never exists (nor, for the difference kind, the (B,K,E,B,K) tensor of differences).  Any other score
 function runs the literal block.
 
-Multi-GPU: one process per GPU.  Each rank trains on its contiguous slice of every batch, negatives stay on
-the rank, gradients are averaged by ``ddp.GradientBucketReducer`` while backward runs.
+Multi-GPU: one process per GPU.  Each rank trains on its contiguous slice of every batch, gradients are averaged by
+``ddp.GradientBucketReducer`` while backward runs.  Negatives stay on the rank unless ``global_negatives=True``, which
+ranks every target against the predictions of the whole global batch, as the reference's nn.DataParallel does
+(``ddp`` module docstring).
 """
 import math
 import time
@@ -60,7 +62,17 @@ class ContrastiveEstimationTrainer:
                  test_task_set=None, prediction_noise=0.01, optimizer=torch.optim.Adam, file_batch_size=1,
                  score_over_all_timesteps=False, score_function=softplus_score_function,
                  wasserstein_gradient_penalty=False, gradient_penalty_factor=10., preprocessing=None, ar_size=256,
-                 prediction_steps=16, verbose=True):
+                 prediction_steps=16, verbose=True, global_negatives=False):
+        """``global_negatives``: with more than one rank, score each rank's targets against the predictions of every
+        rank (the reference's nn.DataParallel objective) instead of its own only; the returned loss and max score are
+        then the global ones on every rank.  Needs a fused score function and no gradient penalty.  validate() keeps
+        per-rank negatives.  No effect on a single rank."""
+        if global_negatives and score_function not in _FUSED_KINDS:
+            raise ValueError("global_negatives needs linear_score_function, softplus_score_function or "
+                             "difference_score_function (the fused kernels)")
+        if global_negatives and wasserstein_gradient_penalty:
+            raise ValueError("global_negatives does not support wasserstein_gradient_penalty: the penalty's sum of "
+                             "scores would need the other ranks' scores")
         self.model = model
         self.ar_size = ar_size
         self.prediction_steps = prediction_steps
@@ -81,6 +93,7 @@ class ContrastiveEstimationTrainer:
         self.gradient_penalty_factor = gradient_penalty_factor
         self.preprocessing = preprocessing
         self.verbose = verbose
+        self.global_negatives = global_negatives
         self.rank, self.world = 0, 1
         if torch.distributed.is_available() and torch.distributed.is_initialized():
             self.rank, self.world = torch.distributed.get_rank(), torch.distributed.get_world_size()
@@ -108,6 +121,13 @@ class ContrastiveEstimationTrainer:
         if self.wasserstein_gradient_penalty:
             return self._loss_with_gradient_penalty(batch, kind)
         predicted_z, targets, _, _ = self.model(batch)
+        if self.global_negatives and self.world > 1:
+            # rank r's shard loss L_r on the gathered predictions; loss / max carry the global values (mean_r L_r,
+            # max_r max_r) and the gradient of L_r (ddp module docstring)
+            loss_r, max_r, _, _ = ops.infonce(ddp.gather_predictions(predicted_z), targets,
+                                              self.score_over_all_timesteps, kind, self.regularization,
+                                              target_offset=self.rank * predicted_z.shape[0])
+            return ddp.combine_shard_losses(loss_r, max_r)
         if kind is not None:
             loss, max_score, _, _ = ops.infonce(predicted_z, targets, self.score_over_all_timesteps, kind,
                                                 self.regularization)

@@ -9,6 +9,9 @@
 // as squared differences in fp32 (tile_dist), never as |p|^2 + |z|^2 - 2 p.z.
 // loss = mean_c (lse_r S[:,c] - S[c,c]) + lambda * mean((mean_k S)^2).  The reference's per-step
 // ".view" scramble is a bijection under the mean, so the training loss equals this clean form.
+// Rectangular problems (cpc_infonce_shard, the shard of a data-parallel rank with the gathered global batch as
+// candidates): P holds pred_batch items, Z holds `batch` items, and the positive of column c sits at row
+// c + doff, doff = target_offset (x K in all-steps mode).  Square calls are pred_batch == batch, doff == 0.
 //
 // Forward : score tiles (64x64) -> per-(row tile, column) partial (max, sum-exp), diagonal, max,
 //           sum, regulariser partials -> combine -> 4 scalars + lse per column.
@@ -21,21 +24,23 @@
 namespace cpc {
 
 // infonce_umma.cu: tcgen05 path (>= 128 candidates per softmax, E % 64 == 0)
-bool nce_umma_eligible(const cpc_infonce_params* p, int which);
-size_t nce_umma_workspace(const cpc_infonce_params* p, int which);
+bool nce_umma_eligible(const cpc_infonce_params* p, const cpc_infonce_shard& sh, int which);
+size_t nce_umma_workspace(const cpc_infonce_params* p, const cpc_infonce_shard& sh, int which);
 int nce_umma_fwd(const float* pred, const float* targets, float* out, float* lse, const cpc_infonce_params* p,
-                 void* workspace, size_t workspace_bytes, cudaStream_t s);
+                 const cpc_infonce_shard& sh, void* workspace, size_t workspace_bytes, cudaStream_t s);
 int nce_umma_bwd(const float* pred, const float* targets, const float* lse, const float* grad_loss, float* d_pred,
-                 float* d_targets, const cpc_infonce_params* p, void* workspace, size_t workspace_bytes, cudaStream_t s);
+                 float* d_targets, const cpc_infonce_params* p, const cpc_infonce_shard& sh, void* workspace,
+                 size_t workspace_bytes, cudaStream_t s);
 
 // flags & CPC_INFONCE_FLAG_NO_TENSOR keeps everything on the CUDA-core kernels (A/B switch for tests)
-static bool nce_tensor_path(const cpc_infonce_params* p, int which) {
+static bool nce_tensor_path(const cpc_infonce_params* p, const cpc_infonce_shard& sh, int which) {
     if (p->flags & CPC_INFONCE_FLAG_NO_TENSOR) return false;
-    return nce_umma_eligible(p, which);
+    return nce_umma_eligible(p, sh, which);
 }
 
 struct NceGeom {
     int B, K, E, all, kind;
+    int Bp, doff;                                 // prediction items; row of column c's positive = c + doff
     int R, C, nprob, tmr, ncols, nrowtiles;
     long long sb, se, sk;
     float lambda;
@@ -51,13 +56,25 @@ static int nce_validate(const cpc_infonce_params* p) {
     return CPC_OK;
 }
 
-static NceGeom nce_geom(const cpc_infonce_params* p) {
+// shard == NULL: the square problem.  Otherwise pred_batch >= batch and 0 <= target_offset <= pred_batch - batch.
+static int nce_validate_shard(const cpc_infonce_params* p, const cpc_infonce_shard* shard, cpc_infonce_shard* out) {
+    *out = cpc_infonce_shard{p->batch, 0};
+    if (!shard) return CPC_OK;
+    if (shard->pred_batch < p->batch || shard->target_offset < 0 || shard->target_offset > shard->pred_batch - p->batch)
+        return CPC_ERR_BAD_SHAPE;
+    if ((int64_t)shard->pred_batch * p->steps > (1 << 30)) return CPC_ERR_BAD_SHAPE;
+    *out = *shard;
+    return CPC_OK;
+}
+
+static NceGeom nce_geom(const cpc_infonce_params* p, const cpc_infonce_shard& sh) {
     NceGeom g;
     g.B = p->batch; g.K = p->steps; g.E = p->enc; g.all = p->all_steps ? 1 : 0; g.kind = p->score_kind;
+    g.Bp = sh.pred_batch;
     g.sb = p->tgt_stride_b; g.se = p->tgt_stride_e; g.sk = p->tgt_stride_k;
     g.lambda = p->regularization;
-    if (g.all) { g.R = g.C = g.B * g.K; g.nprob = 1; g.tmr = (TILE / g.K) * g.K; }
-    else       { g.R = g.C = g.B;       g.nprob = g.K; g.tmr = TILE; }
+    if (g.all) { g.R = g.Bp * g.K; g.C = g.B * g.K; g.nprob = 1; g.tmr = (TILE / g.K) * g.K; g.doff = sh.target_offset * g.K; }
+    else       { g.R = g.Bp;       g.C = g.B;       g.nprob = g.K; g.tmr = TILE; g.doff = sh.target_offset; }
     g.ncols = g.B * g.K;
     g.nrowtiles = ceil_div(g.R, g.tmr);
     return g;
@@ -201,7 +218,7 @@ __global__ void __launch_bounds__(TILE_THREADS) nce_fwd_kernel(const float* __re
                 if (ok[i][j]) {
                     tmax = fmaxf(tmax, v);
                     tsum += v;
-                    if (r == c) diag[prob * g.C + c] = v;
+                    if (r == c + g.doff) diag[prob * g.C + c] = v;
                     if (reg_steps) atomicAdd(rsum + (size_t)r * g.C + c, v);
                 }
             }
@@ -310,8 +327,8 @@ __global__ void __launch_bounds__(256) nce_final_kernel(const float* __restrict_
     rg = block_sum(rg, red);
     if (threadIdx.x == 0) {
         const float loss0 = a / (float)g.ncols;
-        const double nscores = g.all ? (double)g.R * g.C : (double)g.K * g.B * g.B;
-        const double nreg = g.all ? (double)g.B * g.C : (double)g.B * g.B;
+        const double nscores = (double)g.nprob * g.R * g.C;
+        const double nreg = g.all ? (double)g.Bp * g.C : (double)g.R * g.C;   // entries (d, t[, k']) of mean_k S
         out[0] = loss0 + g.lambda * (float)(rg / nreg);
         out[1] = mx;
         out[2] = loss0;
@@ -403,8 +420,8 @@ __global__ void __launch_bounds__(TILE_THREADS) nce_bwd_kernel(const float* __re
     const float gl = __ldg(grad_loss);
     const float inv_k = 1.f / (float)g.K;
     const float w_ce = gl / (float)g.ncols;
-    const float w_reg = g.all ? gl * g.lambda * 2.f * inv_k / ((float)g.B * (float)g.C)
-                              : gl * g.lambda * 2.f * inv_k / ((float)g.B * (float)g.B);
+    const float w_reg = g.all ? gl * g.lambda * 2.f * inv_k / ((float)g.Bp * (float)g.C)
+                              : gl * g.lambda * 2.f * inv_k / ((float)g.Bp * (float)g.B);
     float sbar[4][4] = {};
     if (!g.all && g.lambda != 0.f) {
 #pragma unroll
@@ -459,7 +476,7 @@ __global__ void __launch_bounds__(TILE_THREADS) nce_bwd_kernel(const float* __re
                 float gv = 0.f;
                 if (ok) {
                     const float l = __ldg(lse + (size_t)prob * g.C + c);
-                    gv = w_ce * (expf(s[i][j] - l) - (r == c ? 1.f : 0.f)) + w_reg * sbar[i][j];
+                    gv = w_ce * (expf(s[i][j] - l) - (r == c + g.doff ? 1.f : 0.f)) + w_reg * sbar[i][j];
                     if (kDiff) gv *= 2.f * s[i][j] * s[i][j];
                     else if (g.kind == CPC_SCORE_SOFTPLUS) gv *= sigmoid_f(acc[i][j]);
                 }
@@ -561,14 +578,17 @@ static NceWs nce_ws(const NceGeom& g, void* base) {
 
 using namespace cpc;
 
-extern "C" size_t cpc_infonce_workspace_bytes(const cpc_infonce_params* p, int which) {
-    if (nce_validate(p) != CPC_OK) return 0;
-    const NceGeom g = nce_geom(p);
+// The plain entry points are the _ex ones with shard = NULL (the square problem).
+extern "C" size_t cpc_infonce_workspace_bytes_ex(const cpc_infonce_params* p, const cpc_infonce_shard* shard, int which) {
+    cpc_infonce_shard sh;
+    if (nce_validate(p) != CPC_OK || nce_validate_shard(p, shard, &sh) != CPC_OK) return 0;
+    if (which == 2 && shard) return 0;                         // validation keeps per-rank negatives: no shard
+    const NceGeom g = nce_geom(p, sh);
     if (which == 1)
-        return nce_umma_eligible(p, 1) ? nce_umma_workspace(p, 1) : align_up(sizeof(float) * nce_rsum_floats(g), 256);
+        return nce_umma_eligible(p, sh, 1) ? nce_umma_workspace(p, sh, 1) : align_up(sizeof(float) * nce_rsum_floats(g), 256);
     size_t fwd = nce_ws(g, nullptr).bytes;
     if (which == 0) {
-        if (nce_umma_eligible(p, 0) && nce_umma_workspace(p, 0) > fwd) fwd = nce_umma_workspace(p, 0);
+        if (nce_umma_eligible(p, sh, 0) && nce_umma_workspace(p, sh, 0) > fwd) fwd = nce_umma_workspace(p, sh, 0);
         return fwd;
     }
     // validate: forward scratch + lse + 4 scalars + per-(column tile, row) arg-max partials
@@ -576,17 +596,24 @@ extern "C" size_t cpc_infonce_workspace_bytes(const cpc_infonce_params* p, int w
     return fwd + align_up(sizeof(float) * (size_t)g.ncols, 256) + 256 + 2 * align_up(sizeof(float) * rows, 256);
 }
 
-extern "C" int cpc_infonce_fwd(const float* pred, const float* targets, float* out, float* lse,
-                               const cpc_infonce_params* p, void* workspace, size_t workspace_bytes, void* stream) {
+extern "C" size_t cpc_infonce_workspace_bytes(const cpc_infonce_params* p, int which) {
+    return cpc_infonce_workspace_bytes_ex(p, nullptr, which);
+}
+
+extern "C" int cpc_infonce_fwd_ex(const float* pred, const float* targets, float* out, float* lse,
+                                  const cpc_infonce_params* p, const cpc_infonce_shard* shard, void* workspace,
+                                  size_t workspace_bytes, void* stream) {
     int st = nce_validate(p);
     if (st != CPC_OK) return st;
+    cpc_infonce_shard sh;
+    if ((st = nce_validate_shard(p, shard, &sh)) != CPC_OK) return st;
     if (!pred || !targets || !out || !lse) return CPC_ERR_NULL;
-    NceGeom g = nce_geom(p);
+    NceGeom g = nce_geom(p, sh);
     NceWs w = nce_ws(g, workspace);
-    if (!workspace || workspace_bytes < cpc_infonce_workspace_bytes(p, 0)) return CPC_ERR_WORKSPACE;
+    if (!workspace || workspace_bytes < cpc_infonce_workspace_bytes_ex(p, &sh, 0)) return CPC_ERR_WORKSPACE;
     if ((st = check_device()) != CPC_OK) return st;
     cudaStream_t s = (cudaStream_t)stream;
-    if (nce_tensor_path(p, 0)) return nce_umma_fwd(pred, targets, out, lse, p, workspace, workspace_bytes, s);
+    if (nce_tensor_path(p, sh, 0)) return nce_umma_fwd(pred, targets, out, lse, p, sh, workspace, workspace_bytes, s);
     const size_t n_rsum = nce_rsum_floats(g);
     if (n_rsum && cudaMemsetAsync(w.rsum, 0, sizeof(float) * n_rsum, s) != cudaSuccess) return CPC_ERR_CUDA;
     dim3 grid(ceil_div(g.C, TILE), g.nrowtiles, g.nprob);
@@ -601,22 +628,28 @@ extern "C" int cpc_infonce_fwd(const float* pred, const float* targets, float* o
     return CPC_OK;
 }
 
-extern "C" int cpc_infonce_bwd(const float* pred, const float* targets, const float* lse, const float* grad_loss,
-                               float* d_pred, float* d_targets, const cpc_infonce_params* p, void* workspace,
-                               size_t workspace_bytes, void* stream) {
+extern "C" int cpc_infonce_fwd(const float* pred, const float* targets, float* out, float* lse,
+                               const cpc_infonce_params* p, void* workspace, size_t workspace_bytes, void* stream) {
+    return cpc_infonce_fwd_ex(pred, targets, out, lse, p, nullptr, workspace, workspace_bytes, stream);
+}
+
+extern "C" int cpc_infonce_bwd_ex(const float* pred, const float* targets, const float* lse, const float* grad_loss,
+                                  float* d_pred, float* d_targets, const cpc_infonce_params* p,
+                                  const cpc_infonce_shard* shard, void* workspace, size_t workspace_bytes, void* stream) {
     int st = nce_validate(p);
     if (st != CPC_OK) return st;
+    cpc_infonce_shard sh;
+    if ((st = nce_validate_shard(p, shard, &sh)) != CPC_OK) return st;
     if (!pred || !targets || !lse || !grad_loss || !d_pred || !d_targets) return CPC_ERR_NULL;
     if ((st = check_device()) != CPC_OK) return st;
-    NceGeom g = nce_geom(p);
+    NceGeom g = nce_geom(p, sh);
     cudaStream_t s = (cudaStream_t)stream;
-    if (nce_tensor_path(p, 1)) {
-        if (!workspace || workspace_bytes < nce_umma_workspace(p, 1)) return CPC_ERR_WORKSPACE;
-        return nce_umma_bwd(pred, targets, lse, grad_loss, d_pred, d_targets, p, workspace, workspace_bytes, s);
+    if (nce_tensor_path(p, sh, 1)) {
+        if (!workspace || workspace_bytes < nce_umma_workspace(p, sh, 1)) return CPC_ERR_WORKSPACE;
+        return nce_umma_bwd(pred, targets, lse, grad_loss, d_pred, d_targets, p, sh, workspace, workspace_bytes, s);
     }
-    const size_t n = sizeof(float) * (size_t)g.B * g.K * g.E;
-    if (cudaMemsetAsync(d_pred, 0, n, s) != cudaSuccess) return CPC_ERR_CUDA;
-    if (cudaMemsetAsync(d_targets, 0, n, s) != cudaSuccess) return CPC_ERR_CUDA;
+    if (cudaMemsetAsync(d_pred, 0, sizeof(float) * (size_t)g.Bp * g.K * g.E, s) != cudaSuccess) return CPC_ERR_CUDA;
+    if (cudaMemsetAsync(d_targets, 0, sizeof(float) * (size_t)g.B * g.K * g.E, s) != cudaSuccess) return CPC_ERR_CUDA;
     float* rsum = nullptr;
     if (const size_t n_rsum = nce_rsum_floats(g)) {
         if (!workspace || workspace_bytes < sizeof(float) * n_rsum) return CPC_ERR_WORKSPACE;
@@ -636,6 +669,13 @@ extern "C" int cpc_infonce_bwd(const float* pred, const float* targets, const fl
     return CPC_OK;
 }
 
+extern "C" int cpc_infonce_bwd(const float* pred, const float* targets, const float* lse, const float* grad_loss,
+                               float* d_pred, float* d_targets, const cpc_infonce_params* p, void* workspace,
+                               size_t workspace_bytes, void* stream) {
+    return cpc_infonce_bwd_ex(pred, targets, lse, grad_loss, d_pred, d_targets, p, nullptr, workspace, workspace_bytes,
+                              stream);
+}
+
 extern "C" int cpc_infonce_validate(const float* pred, const float* targets, float* metrics,
                                     const cpc_infonce_params* p, void* workspace, size_t workspace_bytes, void* stream) {
     int st = nce_validate(p);
@@ -644,7 +684,7 @@ extern "C" int cpc_infonce_validate(const float* pred, const float* targets, flo
     const size_t need = cpc_infonce_workspace_bytes(p, 2);
     if (!workspace || workspace_bytes < need) return CPC_ERR_WORKSPACE;
     if ((st = check_device()) != CPC_OK) return st;
-    NceGeom g = nce_geom(p);
+    NceGeom g = nce_geom(p, cpc_infonce_shard{p->batch, 0});
     g.lambda = 0.f;                                            // validation reports the un-regularised loss
     NceWs w = nce_ws(g, workspace);
     char* base = reinterpret_cast<char*>(workspace) + w.bytes;

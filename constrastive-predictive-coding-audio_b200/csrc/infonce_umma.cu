@@ -4,13 +4,17 @@
 // score GEMM dominates (>= 128 candidates per softmax, E a multiple of 64).  Smaller / regularised cases stay on
 // the CUDA-core kernels of infonce.cu, which share the lse layout.
 //
-// Problems: nprob independent (rows x cols) = (Bp x Bp) score matrices over E:
-//   all-steps: nprob = 1, Bp = B*K, prediction row r = (d,k), target column c = (t,k')
-//   per-step : nprob = K, Bp = B,   prediction row d, target column t, one problem per step k
+// Problems: nprob independent (rows x cols) = (Rp x Cp) score matrices over E:
+//   all-steps: nprob = 1, Rp = Bpred*K, Cp = B*K, prediction row r = (d,k), target column c = (t,k')
+//   per-step : nprob = K, Rp = Bpred,   Cp = B,   prediction row d, target column t, one problem per step k
+// Square calls have Bpred = B and the positive of column c at row c; a rectangular call (cpc_infonce_shard: one rank's
+// targets against the gathered global predictions) has Bpred >= B and the positive at row c + doff.
 // Both operands are packed as K-major bf16 hi/lo planes  X[plane][prob][row][E]  (targets are transposed out of
 // their strided (B,E,K) view on the way), fp32-faithful arithmetic = 3 MMAs per product.
 //
-// Forward (nce_umma_fwd_kernel): CTA = (prob, 128 target columns) loops over all 128-row prediction tiles.
+// Forward (nce_umma_fwd_kernel): CTA = (prob, 128 target columns) loops over all 128-row prediction tiles.  A
+//   rectangular call has few column tiles (e24 on 8 GPUs: 8 of them for 64 row tiles), so its row tiles are split over
+//   `rsplit` CTAs: each writes a partial (max, sum-exp) per column and nu_combine_kernel merges them.
 //   D[target c (TMEM lane), prediction r (column)] -- targets sit on M, so the softmax reduction over predictions
 //   is a per-THREAD online max / sum-exp over the accumulator row: no shuffles, no partial buffers; two TMEM
 //   accumulators overlap the reduction of tile i with the MMAs of tile i+1.
@@ -32,23 +36,42 @@ constexpr int NU_BSTAGES = 2;                     // backward ring
 
 struct NuGeom {
     int B, K, E, all, kind;
-    int Bp, nprob, nT, EC;                        // rows per problem, problems, 128-row tiles, 64-wide E chunks
+    int Bpred;                                    // prediction items (B for a square call)
+    int Rp, Cp, nprob, nTr, nTc, EC;              // prediction rows / target columns per problem, problems, their 128-row
+                                                  // tiles, 64-wide E chunks
+    int doff;                                     // prediction row of target column c's positive: c + doff
+    int rsplit;                                   // forward CTAs per (problem, column tile), each a range of row tiles
     int passes;                                   // MMA passes per product: 3 = fp32-faithful (hi*hi + hi*lo + lo*hi),
                                                   // 1 = bf16 operand mode (precision = 1: the hi planes only)
     float lambda;
 };
 
-static NuGeom nu_geom(const cpc_infonce_params* p) {
+static NuGeom nu_geom(const cpc_infonce_params* p, const cpc_infonce_shard& sh) {
     NuGeom g;
     g.B = p->batch; g.K = p->steps; g.E = p->enc; g.all = p->all_steps ? 1 : 0; g.kind = p->score_kind;
-    g.Bp = g.all ? g.B * g.K : g.B;
+    g.Bpred = sh.pred_batch;
+    g.Rp = g.all ? g.Bpred * g.K : g.Bpred;
+    g.Cp = g.all ? g.B * g.K : g.B;
+    g.doff = g.all ? sh.target_offset * g.K : sh.target_offset;
     g.nprob = g.all ? 1 : g.K;
-    g.nT = ceil_div(g.Bp, 128);
+    g.nTr = ceil_div(g.Rp, 128);
+    g.nTc = ceil_div(g.Cp, 128);
     g.EC = g.E / 64;
+    // square calls: one CTA per column tile loops over every row tile (no partial buffers).  Rectangular: enough CTAs
+    // for the 148 SMs, at least one row tile each
+    g.rsplit = 1;
+    if (g.Bpred != g.B || g.doff != 0) {
+        g.rsplit = 148 / (g.nprob * g.nTc);
+        if (g.rsplit > g.nTr) g.rsplit = g.nTr;
+        if (g.rsplit < 1) g.rsplit = 1;
+    }
     g.lambda = p->regularization;
     g.passes = p->precision == 0 ? 3 : 1;
     return g;
 }
+
+// a rectangular call (kernels instantiated with RECT = true); square calls keep the square kernels
+static bool nu_rect(const NuGeom& g) { return g.Bpred != g.B || g.doff != 0; }
 
 // src element (prob, row, e) at base + prob*sp + row_major*s1 + row_minor*s2 + e*se, row = row_major*minor + row_minor
 struct NuSrc { const float* p; long long sp, s1, s2, se; int minor; };
@@ -95,17 +118,26 @@ struct __align__(8) NuFwdBarriers {
     float red[4][4];
 };
 
-// per-CTA partials: [cta][0] sum over its columns of (lse - diag), [1] max score, [2] sum of scores, [3] regulariser
-template <int KIND, bool REG>
+// RECT = false: square calls, the code and grid of square problems before rectangles existed (positive of column c at
+// row c, one CTA per column tile).  RECT = true: rectangles, positive at row c + doff, optional row split.
+// per-CTA partials: [cta][0] sum over its columns of (lse - diag), [1] max score, [2] sum of scores, [3] regulariser.
+// Row split (g.rsplit > 1): [cta][0] = 0; per column, part_m / part_s [split][prob * Cp + c] get this CTA's (max, sum-exp)
+// and diag [prob * Cp + c] the positive's score (from the CTA whose rows hold it); nu_combine_kernel forms lse.
+template <int KIND, bool REG, bool RECT>
 __global__ void __launch_bounds__(NU_THREADS, 1) nce_umma_fwd_kernel(const __grid_constant__ CUtensorMap tmap_z,
                                                                     const __grid_constant__ CUtensorMap tmap_p,
                                                                     const NuGeom g, float* __restrict__ lse,
-                                                                    float* __restrict__ partials) {
+                                                                    float* __restrict__ partials,
+                                                                    float* __restrict__ part_m, float* __restrict__ part_s,
+                                                                    float* __restrict__ diag_out) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
     NuFwdBarriers* bars = reinterpret_cast<NuFwdBarriers*>(smem + NU_FSTAGES * 2 * NU_TILE);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int prob = blockIdx.x / g.nT, ct = blockIdx.x - prob * g.nT;
+    const int rs = RECT ? blockIdx.x % g.rsplit : 0, pc = RECT ? blockIdx.x / g.rsplit : blockIdx.x;
+    const int prob = pc / g.nTc, ct = pc - prob * g.nTc;
+    const int rt0 = RECT ? (int)((long)rs * g.nTr / g.rsplit) : 0;                       // this CTA's row tiles
+    const int rt1 = RECT ? (int)((long)(rs + 1) * g.nTr / g.rsplit) : g.nTr;
 
     if (warp == 0 && lane == 0) {
         prefetch_tmap(&tmap_z);
@@ -123,7 +155,7 @@ __global__ void __launch_bounds__(NU_THREADS, 1) nce_umma_fwd_kernel(const __gri
     if (warp == 0) {
         if (lane == 0) {
             uint32_t n = 0;
-            for (int rt = 0; rt < g.nT; ++rt)
+            for (int rt = rt0; rt < rt1; ++rt)
                 for (int q = 0; q < g.EC; ++q, ++n) {
                     const int stage = n % NU_FSTAGES;
                     mbar_wait(&bars->empty[stage], ((n / NU_FSTAGES) & 1) ^ 1);
@@ -137,9 +169,9 @@ __global__ void __launch_bounds__(NU_THREADS, 1) nce_umma_fwd_kernel(const __gri
         if (lane == 0) {
             const uint32_t idesc = make_idesc_bf16(128, 128, 0, 0);
             uint32_t n = 0;
-            for (int rt = 0; rt < g.nT; ++rt) {
-                const uint32_t buf = rt & 1;
-                mbar_wait(&bars->acc_empty[buf], ((rt >> 1) & 1) ^ 1);
+            for (int it = 0; it < rt1 - rt0; ++it) {
+                const uint32_t buf = it & 1;
+                mbar_wait(&bars->acc_empty[buf], ((it >> 1) & 1) ^ 1);
                 tc_fence_after();
                 const uint32_t d_tmem = tmem_base + buf * 128;
                 for (int q = 0; q < g.EC; ++q, ++n) {
@@ -166,15 +198,16 @@ __global__ void __launch_bounds__(NU_THREADS, 1) nce_umma_fwd_kernel(const __gri
         const int ew = warp & 3;
         const int cl = ew * 32 + lane;
         const int c = ct * 128 + cl;
-        const bool col_ok = c < g.Bp;
+        const int prow = c + g.doff;                                         // prediction row of this column's positive
+        const bool col_ok = c < g.Cp;
         float m = -INFINITY, ssum = 0.f, diag = 0.f, vmax = -INFINITY, vsum = 0.f, reg = 0.f, grp = 0.f;
         const float inv_k = 1.f / (float)g.K;
-        for (int rt = 0; rt < g.nT; ++rt) {
-            const uint32_t buf = rt & 1;
-            mbar_wait(&bars->acc_full[buf], (rt >> 1) & 1);
+        for (int rt = rt0; rt < rt1; ++rt) {
+            const uint32_t buf = (rt - rt0) & 1;
+            mbar_wait(&bars->acc_full[buf], ((rt - rt0) >> 1) & 1);
             tc_fence_after();
             const uint32_t taddr = tmem_base + ((uint32_t)(ew * 32) << 16) + buf * 128;
-            const int n_valid = min(128, g.Bp - rt * 128);                   // prediction rows of this tile inside the problem
+            const int n_valid = min(128, g.Rp - rt * 128);                   // prediction rows of this tile inside the problem
             for (int n0 = 0; n0 < 128; n0 += 32) {
                 uint32_t raw[32];
                 tmem_ld32(taddr + n0, raw);
@@ -190,7 +223,13 @@ __global__ void __launch_bounds__(NU_THREADS, 1) nce_umma_fwd_kernel(const __gri
 #pragma unroll
                     for (int j = 0; j < 32; ++j) if (n0 + j >= n_valid) v[j] = -INFINITY;
                 }
-                if (rt == ct && n0 == (cl & 96)) {                           // the tile on the diagonal holds S[c, c]
+                if (RECT) {   // the chunk holding S[c + doff, c]; a select per j keeps v[] in registers (an index taken
+                              // from prow inside a branch made the compiler move v[] to the stack)
+                    const bool here = rt == (prow >> 7) && n0 == (prow & 96);
+                    const int jj = prow & 31;
+#pragma unroll
+                    for (int j = 0; j < 32; ++j) diag = (here && j == jj) ? v[j] : diag;
+                } else if (rt == ct && n0 == (cl & 96)) {                    // the tile on the diagonal holds S[c, c]
 #pragma unroll
                     for (int j = 0; j < 32; ++j) if (j == (cl & 31)) diag = v[j];
                 }
@@ -221,9 +260,16 @@ __global__ void __launch_bounds__(NU_THREADS, 1) nce_umma_fwd_kernel(const __gri
         }
         float term = 0.f;
         if (col_ok) {
-            const float l = m + logf(ssum);
-            lse[(size_t)prob * g.Bp + c] = l;
-            term = l - diag;
+            if (RECT && part_m != nullptr) {
+                const size_t o = (size_t)prob * g.Cp + c;
+                part_m[(size_t)rs * g.nprob * g.Cp + o] = m;
+                part_s[(size_t)rs * g.nprob * g.Cp + o] = ssum;
+                if ((prow >> 7) >= rt0 && (prow >> 7) < rt1) diag_out[o] = diag;
+            } else {
+                const float l = m + logf(ssum);
+                lse[(size_t)prob * g.Cp + c] = l;
+                term = l - diag;
+            }
         }
         term = warp_sum(term);
         vmax = warp_max(vmax);
@@ -242,6 +288,34 @@ __global__ void __launch_bounds__(NU_THREADS, 1) nce_umma_fwd_kernel(const __gri
     tc_fence_before();
     __syncthreads();
     if (warp == 2) { tc_fence_after(); tmem_dealloc(tmem_base, 256); }
+}
+
+// Row split: one thread per column merges the splits' (max, sum-exp) into lse; each block appends one 4-float partial
+// {sum of (lse - diag), -inf, 0, 0} behind the CTA partials for nce_umma_final_kernel.
+__global__ void __launch_bounds__(256) nu_combine_kernel(const float* __restrict__ part_m, const float* __restrict__ part_s,
+                                                        const float* __restrict__ diag, float* __restrict__ lse,
+                                                        float* __restrict__ partials, int ncols, int nsplit) {
+    __shared__ float red[8];
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    float term = 0.f;
+    if (c < ncols) {
+        float m = -INFINITY;
+        for (int t = 0; t < nsplit; ++t) m = fmaxf(m, part_m[(size_t)t * ncols + c]);
+        float s = 0.f;
+        for (int t = 0; t < nsplit; ++t) s += part_s[(size_t)t * ncols + c] * expf(part_m[(size_t)t * ncols + c] - m);
+        const float l = m + logf(s);
+        lse[c] = l;
+        term = l - diag[c];
+    }
+    term = warp_sum(term);
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = term;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float a = 0.f;
+        for (int w = 0; w < 8; ++w) a += red[w];
+        float* o = partials + (size_t)blockIdx.x * 4;
+        o[0] = a; o[1] = -INFINITY; o[2] = 0.f; o[3] = 0.f;
+    }
 }
 
 // out[0] loss, [1] max score, [2] loss without regulariser, [3] mean score
@@ -263,9 +337,9 @@ __global__ void __launch_bounds__(256) nce_umma_final_kernel(const float* __rest
     if (threadIdx.x == 0) {
         a = 0.f; mx = -INFINITY; sm = 0.f; rg = 0.f;
         for (int w = 0; w < 8; ++w) { a += red[0][w]; mx = fmaxf(mx, red[1][w]); sm += red[2][w]; rg += red[3][w]; }
-        const double ncols = (double)g.nprob * g.Bp;
-        const double nscores = (double)g.nprob * g.Bp * g.Bp;
-        const double nreg = g.all ? (double)g.B * g.Bp : (double)g.B * g.B;
+        const double ncols = (double)g.nprob * g.Cp;
+        const double nscores = (double)g.nprob * g.Rp * g.Cp;
+        const double nreg = g.all ? (double)g.Bpred * g.Cp : (double)g.Rp * g.Cp;   // entries (d, t[, k']) of mean_k S
         const float loss0 = (float)(a / ncols);
         out[0] = loss0 + g.lambda * (float)(rg / nreg);
         out[1] = mx;
@@ -287,12 +361,14 @@ struct NuBwd {
     int n_slices;                 // E / 256 (ceil)
     int n_split;                  // CTAs sharing one (problem, owner tile, E slice): each takes a range of the other operand's
                                   // tiles and adds its partial result atomically (small problems: 16 CTAs -> up to 148)
-    const float* lse;             // [prob * Bp + target]
+    int own_rows, oth_rows;       // rows per problem of the owner / other operand (Cp or Rp)
+    int n_own, n_oth;             // their 128-row tiles
+    const float* lse;             // [prob * Cp + target]
     const float* grad_loss;
     float* out;                   // d_targets (B,E,K) contiguous or d_pred (B,K,E) contiguous
 };
 
-template <int KIND>
+template <int KIND, bool RECT>                     // RECT as in the forward: false = square calls' code
 __global__ void __launch_bounds__(NU_THREADS, 1) nce_umma_bwd_kernel(const __grid_constant__ CUtensorMap tmap_owner,
                                                                     const __grid_constant__ CUtensorMap tmap_other,
                                                                     const NuBwd p) {
@@ -306,9 +382,9 @@ __global__ void __launch_bounds__(NU_THREADS, 1) nce_umma_bwd_kernel(const __gri
     int w = blockIdx.x;
     const int es = w % p.n_slices; w /= p.n_slices;
     const int sp = w % p.n_split; w /= p.n_split;
-    const int ot = w % g.nT;
-    const int prob = w / g.nT;
-    const int st0 = (int)((long)sp * g.nT / p.n_split), st1 = (int)((long)(sp + 1) * g.nT / p.n_split);   // other tiles of this CTA
+    const int ot = w % p.n_own;
+    const int prob = w / p.n_own;
+    const int st0 = (int)((long)sp * p.n_oth / p.n_split), st1 = (int)((long)(sp + 1) * p.n_oth / p.n_split);   // other tiles of this CTA
     const int n_it = st1 - st0;
     const int e_chunks = min(4, g.EC - es * 4);                   // 64-wide E chunks in this slice
 
@@ -415,22 +491,23 @@ __global__ void __launch_bounds__(NU_THREADS, 1) nce_umma_bwd_kernel(const __gri
         const int ew = warp & 3;
         const int rl = ew * 32 + lane;                                       // owner row inside the tile
         const int orow = ot * 128 + rl;
-        const bool own_ok = orow < g.Bp;
-        const float w_ce = __ldg(p.grad_loss) / ((float)g.nprob * (float)g.Bp);
-        const float lse_own = (p.owner_is_target && own_ok) ? __ldg(p.lse + (size_t)prob * g.Bp + orow) : 0.f;
+        const bool own_ok = orow < p.own_rows;
+        const int prow = p.owner_is_target ? orow + g.doff : orow - g.doff;  // other row of this owner row's positive pair
+        const float w_ce = __ldg(p.grad_loss) / ((float)g.nprob * (float)g.Cp);
+        const float lse_own = (p.owner_is_target && own_ok) ? __ldg(p.lse + (size_t)prob * g.Cp + orow) : 0.f;
         const uint32_t lane_base = tmem_base + ((uint32_t)(ew * 32) << 16);
         uint8_t* grow = gs + (rl >> 3) * 1024 + (rl & 7) * 128;              // this owner row inside a K atom
         for (int it = 0; it < n_it; ++it) {
             const int st = st0 + it;
             if (!p.owner_is_target) {                                        // lse of the 128 target columns of this tile
                 const int c = st * 128 + rl;
-                bars->lse_s[it & 1][rl] = c < g.Bp ? __ldg(p.lse + (size_t)prob * g.Bp + c) : 0.f;
+                bars->lse_s[it & 1][rl] = c < g.Cp ? __ldg(p.lse + (size_t)prob * g.Cp + c) : 0.f;
             }
             mbar_wait(&bars->s_full[it & 1], (it >> 1) & 1);
             tc_fence_after();
             mbar_wait(&bars->g_empty, (it & 1) ^ 1);                         // previous G tile consumed by the MMAs
             asm volatile("bar.sync 1, 128;" ::: "memory");                  // lse_s visible to all epilogue threads
-            const int n_valid = min(128, g.Bp - st * 128);                   // rows of the other operand inside the problem
+            const int n_valid = min(128, p.oth_rows - st * 128);             // rows of the other operand inside the problem
             const float* lrow = bars->lse_s[it & 1];
             for (int n0 = 0; n0 < 128; n0 += 32) {
                 uint32_t raw[32];
@@ -452,7 +529,7 @@ __global__ void __launch_bounds__(NU_THREADS, 1) nce_umma_bwd_kernel(const __gri
                     // dL/dS[d,k,t,k'] += 2 lambda / (B^2 K^3) * sum_k S[d,k,t,k'].  Prediction rows are ordered (d, k), so the
                     // K-sum runs over K consecutive columns (owner = targets: inside this thread's registers) or over K
                     // consecutive lanes (owner = predictions: warp shuffles); K is a power of two <= 32 (host side).
-                    const float w_reg = __ldg(p.grad_loss) * 2.f * g.lambda / ((float)g.B * (float)g.B * (float)g.K * (float)g.K * (float)g.K);
+                    const float w_reg = __ldg(p.grad_loss) * 2.f * g.lambda / ((float)g.Bpred * (float)g.B * (float)g.K * (float)g.K * (float)g.K);
                     float sc[32];
 #pragma unroll
                     for (int j = 0; j < 32; ++j) {
@@ -484,7 +561,12 @@ __global__ void __launch_bounds__(NU_THREADS, 1) nce_umma_bwd_kernel(const __gri
 #pragma unroll
                     for (int j = 0; j < 32; ++j) gv[j] = fmaf(w_reg, sc[j], gv[j]);
                 }
-                if (st == ot && n0 == (rl & 96)) {                           // - w on the diagonal element
+                if (RECT) {   // - w on the positive pair (prow < 0: none); selects, not a branch on an index (forward)
+                    const bool here = st == (prow >> 7) && n0 == (prow & 96);
+                    const int jj = prow & 31;
+#pragma unroll
+                    for (int j = 0; j < 32; ++j) gv[j] -= (here && j == jj) ? w_ce : 0.f;
+                } else if (st == ot && n0 == (rl & 96)) {                    // - w on the diagonal element
 #pragma unroll
                     for (int j = 0; j < 32; ++j) if (j == (rl & 31)) gv[j] -= w_ce;
                 }
@@ -560,16 +642,21 @@ __global__ void __launch_bounds__(NU_THREADS, 1) nce_umma_bwd_kernel(const __gri
 
 // ---- host side ----------------------------------------------------------------------------------------------
 // which: 0 forward, 1 backward
-bool nce_umma_eligible(const cpc_infonce_params* p, int which) {
+bool nce_umma_eligible(const cpc_infonce_params* p, const cpc_infonce_shard& sh, int which) {
     // the kernels below compute dot products only (any other kind would run as linear), and a distance from them would
     // be |p|^2 + |z|^2 - 2 p.z, which cancels for the near pairs the difference kind is about
     if (p->score_kind == CPC_SCORE_DIFFERENCE) return false;
     if (p->enc % 64 != 0 || p->enc < 64 || p->enc > 4096) return false;
-    const long bp = p->all_steps ? (long)p->batch * p->steps : p->batch;
-    if (bp < 128 || bp > (1 << 24)) return false;                          // tiny problems are latency-bound either way
-    // one CTA per 128 owner rows: a single all-steps problem needs >= 8 row tiles to beat
-    // the CUDA-core kernel does (measured cross-over, tools/infonce_sweep.py); per-step mode has K problems
-    if (p->all_steps && bp < 1024) return false;
+    // cols: target columns per problem (the softmax columns, the owner rows of the dZ pass); rows: prediction rows per
+    // problem (the candidates of each softmax).  Square calls have rows == cols.  The rule is stated on the columns,
+    // the rectangle's own batch: the row split spreads a rectangle's forward over the SMs, and the backward's dP pass
+    // has at least as many owner tiles as the dZ pass.
+    const long cols = p->all_steps ? (long)p->batch * p->steps : p->batch;
+    const long rows = p->all_steps ? (long)sh.pred_batch * p->steps : sh.pred_batch;
+    if (cols < 128 || rows > (1 << 24)) return false;                      // tiny problems are latency-bound either way
+    // one CTA per 128 owner rows: a single all-steps problem needs >= 8 column tiles to beat
+    // the CUDA-core kernel does (measured cross-over of square calls, tools/infonce_sweep.py); per-step mode has K problems
+    if (p->all_steps && cols < 1024) return false;
     if (p->regularization != 0.f) {
         if (!p->all_steps || 128 % p->steps != 0) return false;            // whole K-groups inside a tile (K a power of two)
         if (which == 1 && p->steps > 32) return false;                     // backward sums K consecutive lanes with shuffles
@@ -577,12 +664,29 @@ bool nce_umma_eligible(const cpc_infonce_params* p, int which) {
     return true;
 }
 
-static size_t nu_plane_bytes(const NuGeom& g) { return align_up((size_t)2 * g.nprob * g.Bp * g.E * 2, 1024); }
+// one operand's bf16 hi/lo planes, [plane][prob][row][E]
+static size_t nu_plane_bytes(const NuGeom& g, int rows) { return align_up((size_t)2 * g.nprob * rows * g.E * 2, 1024); }
+// forward scratch behind the planes: CTA partials + combine partials (4 floats each), then the row split's per-column
+// (max, sum-exp) of every split and the positives' scores
+struct NuFwdWs { size_t partials, part_m, part_s, diag, bytes; int ncta, nblk; };
+static NuFwdWs nu_fwd_ws(const NuGeom& g) {
+    NuFwdWs w;
+    const size_t ncols = (size_t)g.nprob * g.Cp;
+    w.ncta = g.nprob * g.nTc * g.rsplit;
+    w.nblk = g.rsplit > 1 ? (int)ceil_div((int)ncols, 256) : 0;
+    size_t o = nu_plane_bytes(g, g.Rp) + nu_plane_bytes(g, g.Cp);
+    w.partials = o; o += align_up((size_t)(w.ncta + w.nblk) * 4 * sizeof(float), 256);
+    w.part_m = o; o += g.rsplit > 1 ? align_up((size_t)g.rsplit * ncols * sizeof(float), 256) : 0;
+    w.part_s = o; o += g.rsplit > 1 ? align_up((size_t)g.rsplit * ncols * sizeof(float), 256) : 0;
+    w.diag = o; o += g.rsplit > 1 ? align_up(ncols * sizeof(float), 256) : 0;
+    w.bytes = o;
+    return w;
+}
 
-size_t nce_umma_workspace(const cpc_infonce_params* p, int which) {
-    if (!nce_umma_eligible(p, which)) return 0;
-    const NuGeom g = nu_geom(p);
-    return 2 * nu_plane_bytes(g) + (which == 0 ? align_up((size_t)g.nprob * g.nT * 4 * sizeof(float), 256) : 0) + 2048;
+size_t nce_umma_workspace(const cpc_infonce_params* p, const cpc_infonce_shard& sh, int which) {
+    if (!nce_umma_eligible(p, sh, which)) return 0;
+    const NuGeom g = nu_geom(p, sh);
+    return (which == 0 ? nu_fwd_ws(g).bytes : nu_plane_bytes(g, g.Rp) + nu_plane_bytes(g, g.Cp)) + 2048;
 }
 
 static int nu_pack_both(const float* pred, const float* targets, const cpc_infonce_params* p, const NuGeom& g,
@@ -595,87 +699,114 @@ static int nu_pack_both(const float* pred, const float* targets, const cpc_infon
         sp = NuSrc{pred, (long long)g.E, (long long)g.K * g.E, 0, 1, 1};
         sz = NuSrc{targets, p->tgt_stride_k, p->tgt_stride_b, 0, p->tgt_stride_e, 1};
     }
-    const long groups = (long)g.nprob * g.Bp * (g.E / 8);
-    int blocks = (int)((groups + 255) / 256);
-    if (blocks > 148 * 16) blocks = 148 * 16;
-    nu_pack_kernel<<<blocks, 256, 0, s>>>(sp, pp, g.nprob, g.Bp, g.E);
-    nu_pack_kernel<<<blocks, 256, 0, s>>>(sz, zp, g.nprob, g.Bp, g.E);
+    auto blocks = [&](int rows) {
+        const long groups = (long)g.nprob * rows * (g.E / 8);
+        const long b = (groups + 255) / 256;
+        return (int)(b > 148 * 16 ? 148 * 16 : b);
+    };
+    nu_pack_kernel<<<blocks(g.Rp), 256, 0, s>>>(sp, pp, g.nprob, g.Rp, g.E);
+    nu_pack_kernel<<<blocks(g.Cp), 256, 0, s>>>(sz, zp, g.nprob, g.Cp, g.E);
     return cudaGetLastError() == cudaSuccess ? CPC_OK : CPC_ERR_CUDA;
 }
 
-static bool nu_tmap(CUtensorMap* t, const void* base, const NuGeom& g) {
-    const uint64_t dims[4] = {(uint64_t)g.E, (uint64_t)g.Bp, (uint64_t)g.nprob, 2};
-    const uint64_t strides[3] = {(uint64_t)g.E * 2, (uint64_t)g.Bp * g.E * 2, (uint64_t)g.nprob * g.Bp * g.E * 2};
+static bool nu_tmap(CUtensorMap* t, const void* base, const NuGeom& g, int rows) {
+    const uint64_t dims[4] = {(uint64_t)g.E, (uint64_t)rows, (uint64_t)g.nprob, 2};
+    const uint64_t strides[3] = {(uint64_t)g.E * 2, (uint64_t)rows * g.E * 2, (uint64_t)g.nprob * rows * g.E * 2};
     const uint32_t box[4] = {64, 128, 1, 2};
     return make_tmap_bf16(t, base, 4, dims, strides, box);
 }
 
 int nce_umma_fwd(const float* pred, const float* targets, float* out, float* lse, const cpc_infonce_params* p,
-                 void* workspace, size_t workspace_bytes, cudaStream_t s) {
-    if (!nce_umma_eligible(p, 0)) return CPC_ERR_UNSUPPORTED;
-    if (!workspace || workspace_bytes < nce_umma_workspace(p, 0)) return CPC_ERR_WORKSPACE;
-    const NuGeom g = nu_geom(p);
+                 const cpc_infonce_shard& sh, void* workspace, size_t workspace_bytes, cudaStream_t s) {
+    if (!nce_umma_eligible(p, sh, 0)) return CPC_ERR_UNSUPPORTED;
+    if (!workspace || workspace_bytes < nce_umma_workspace(p, sh, 0)) return CPC_ERR_WORKSPACE;
+    const NuGeom g = nu_geom(p, sh);
+    const NuFwdWs w = nu_fwd_ws(g);
     uint8_t* ws = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(workspace) + 1023) & ~(uintptr_t)1023);
     __nv_bfloat16* pp = reinterpret_cast<__nv_bfloat16*>(ws);
-    __nv_bfloat16* zp = reinterpret_cast<__nv_bfloat16*>(ws + nu_plane_bytes(g));
-    float* partials = reinterpret_cast<float*>(ws + 2 * nu_plane_bytes(g));
+    __nv_bfloat16* zp = reinterpret_cast<__nv_bfloat16*>(ws + nu_plane_bytes(g, g.Rp));
+    float* partials = reinterpret_cast<float*>(ws + w.partials);
+    const bool split = g.rsplit > 1;
+    float* part_m = split ? reinterpret_cast<float*>(ws + w.part_m) : nullptr;
+    float* part_s = split ? reinterpret_cast<float*>(ws + w.part_s) : nullptr;
+    float* diag = split ? reinterpret_cast<float*>(ws + w.diag) : nullptr;
     int st = nu_pack_both(pred, targets, p, g, pp, zp, s);
     if (st != CPC_OK) return st;
     CUtensorMap tz, tp;
-    if (!nu_tmap(&tz, zp, g) || !nu_tmap(&tp, pp, g)) return CPC_ERR_CUDA;
+    if (!nu_tmap(&tz, zp, g, g.Cp) || !nu_tmap(&tp, pp, g, g.Rp)) return CPC_ERR_CUDA;
     const int smem_bytes = NU_FSTAGES * 2 * NU_TILE + (int)sizeof(NuFwdBarriers) + 1024;
-    const int ncta = g.nprob * g.nT;
     auto launch = [&](auto kern) -> int {
         if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes) != cudaSuccess) return CPC_ERR_CUDA;
-        kern<<<ncta, NU_THREADS, smem_bytes, s>>>(tz, tp, g, lse, partials);
+        kern<<<w.ncta, NU_THREADS, smem_bytes, s>>>(tz, tp, g, lse, partials, part_m, part_s, diag);
         return CPC_OK;
     };
     const bool soft = g.kind == CPC_SCORE_SOFTPLUS, reg = g.lambda != 0.f;
-    st = soft ? (reg ? launch(nce_umma_fwd_kernel<CPC_SCORE_SOFTPLUS, true>) : launch(nce_umma_fwd_kernel<CPC_SCORE_SOFTPLUS, false>))
-              : (reg ? launch(nce_umma_fwd_kernel<CPC_SCORE_LINEAR, true>) : launch(nce_umma_fwd_kernel<CPC_SCORE_LINEAR, false>));
+    if (!nu_rect(g))
+        st = soft ? (reg ? launch(nce_umma_fwd_kernel<CPC_SCORE_SOFTPLUS, true, false>)
+                         : launch(nce_umma_fwd_kernel<CPC_SCORE_SOFTPLUS, false, false>))
+                  : (reg ? launch(nce_umma_fwd_kernel<CPC_SCORE_LINEAR, true, false>)
+                         : launch(nce_umma_fwd_kernel<CPC_SCORE_LINEAR, false, false>));
+    else
+        st = soft ? (reg ? launch(nce_umma_fwd_kernel<CPC_SCORE_SOFTPLUS, true, true>)
+                         : launch(nce_umma_fwd_kernel<CPC_SCORE_SOFTPLUS, false, true>))
+                  : (reg ? launch(nce_umma_fwd_kernel<CPC_SCORE_LINEAR, true, true>)
+                         : launch(nce_umma_fwd_kernel<CPC_SCORE_LINEAR, false, true>));
     if (st != CPC_OK) return st;
     CPC_LAUNCH_CHECK();
-    nce_umma_final_kernel<<<1, 256, 0, s>>>(partials, ncta, g, out);
+    if (split) {
+        nu_combine_kernel<<<w.nblk, 256, 0, s>>>(part_m, part_s, diag, lse, partials + (size_t)w.ncta * 4,
+                                                 g.nprob * g.Cp, g.rsplit);
+        CPC_LAUNCH_CHECK();
+    }
+    nce_umma_final_kernel<<<1, 256, 0, s>>>(partials, w.ncta + w.nblk, g, out);
     CPC_LAUNCH_CHECK();
-    count_launch(4);
+    count_launch(split ? 5 : 4);
     return CPC_OK;
 }
 
 int nce_umma_bwd(const float* pred, const float* targets, const float* lse, const float* grad_loss, float* d_pred,
-                 float* d_targets, const cpc_infonce_params* p, void* workspace, size_t workspace_bytes, cudaStream_t s) {
-    if (!nce_umma_eligible(p, 1)) return CPC_ERR_UNSUPPORTED;
-    if (!workspace || workspace_bytes < nce_umma_workspace(p, 1)) return CPC_ERR_WORKSPACE;
-    const NuGeom g = nu_geom(p);
+                 float* d_targets, const cpc_infonce_params* p, const cpc_infonce_shard& sh, void* workspace,
+                 size_t workspace_bytes, cudaStream_t s) {
+    if (!nce_umma_eligible(p, sh, 1)) return CPC_ERR_UNSUPPORTED;
+    if (!workspace || workspace_bytes < nce_umma_workspace(p, sh, 1)) return CPC_ERR_WORKSPACE;
+    const NuGeom g = nu_geom(p, sh);
     uint8_t* ws = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(workspace) + 1023) & ~(uintptr_t)1023);
     __nv_bfloat16* pp = reinterpret_cast<__nv_bfloat16*>(ws);
-    __nv_bfloat16* zp = reinterpret_cast<__nv_bfloat16*>(ws + nu_plane_bytes(g));
+    __nv_bfloat16* zp = reinterpret_cast<__nv_bfloat16*>(ws + nu_plane_bytes(g, g.Rp));
     int st = nu_pack_both(pred, targets, p, g, pp, zp, s);
     if (st != CPC_OK) return st;
     CUtensorMap tz, tp;
-    if (!nu_tmap(&tz, zp, g) || !nu_tmap(&tp, pp, g)) return CPC_ERR_CUDA;
+    if (!nu_tmap(&tz, zp, g, g.Cp) || !nu_tmap(&tp, pp, g, g.Rp)) return CPC_ERR_CUDA;
     const int smem_bytes = NU_BSTAGES * 2 * NU_TILE + 2 * NU_TILE + (int)sizeof(NuBwdBarriers) + 1024;
     NuBwd k{};
     k.g = g; k.lse = lse; k.grad_loss = grad_loss;
     k.n_slices = ceil_div(g.EC, 4);
     // small problems (the native e24 size is 16 CTAs): split the loop over the other operand's tiles across CTAs
-    k.n_split = 148 / (g.nprob * g.nT * k.n_slices);
-    if (k.n_split > g.nT) k.n_split = g.nT;
-    if (k.n_split < 1) k.n_split = 1;
-    const int grid = g.nprob * g.nT * k.n_split * k.n_slices;
-    if (k.n_split > 1) {
-        const size_t n_out = (size_t)g.B * g.K * g.E;
-        if (cudaMemsetAsync(d_targets, 0, n_out * sizeof(float), s) != cudaSuccess ||
-            cudaMemsetAsync(d_pred, 0, n_out * sizeof(float), s) != cudaSuccess) return CPC_ERR_CUDA;
-    }
+    auto n_split = [&](int n_own, int n_oth) {
+        int n = 148 / (g.nprob * n_own * k.n_slices);
+        if (n > n_oth) n = n_oth;
+        return n < 1 ? 1 : n;
+    };
+    const int split_z = n_split(g.nTc, g.nTr), split_p = n_split(g.nTr, g.nTc);   // owner = targets / predictions
+    if ((split_z > 1 && cudaMemsetAsync(d_targets, 0, (size_t)g.B * g.K * g.E * sizeof(float), s) != cudaSuccess) ||
+        (split_p > 1 && cudaMemsetAsync(d_pred, 0, (size_t)g.Bpred * g.K * g.E * sizeof(float), s) != cudaSuccess))
+        return CPC_ERR_CUDA;
     auto launch = [&](auto kern) -> int {
         if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes) != cudaSuccess) return CPC_ERR_CUDA;
         k.owner_is_target = 1; k.out = d_targets;
-        kern<<<grid, NU_THREADS, smem_bytes, s>>>(tz, tp, k);
+        k.own_rows = g.Cp; k.oth_rows = g.Rp; k.n_own = g.nTc; k.n_oth = g.nTr; k.n_split = split_z;
+        kern<<<g.nprob * g.nTc * split_z * k.n_slices, NU_THREADS, smem_bytes, s>>>(tz, tp, k);
         k.owner_is_target = 0; k.out = d_pred;
-        kern<<<grid, NU_THREADS, smem_bytes, s>>>(tp, tz, k);
+        k.own_rows = g.Rp; k.oth_rows = g.Cp; k.n_own = g.nTr; k.n_oth = g.nTc; k.n_split = split_p;
+        kern<<<g.nprob * g.nTr * split_p * k.n_slices, NU_THREADS, smem_bytes, s>>>(tp, tz, k);
         return CPC_OK;
     };
-    st = g.kind == CPC_SCORE_SOFTPLUS ? launch(nce_umma_bwd_kernel<CPC_SCORE_SOFTPLUS>) : launch(nce_umma_bwd_kernel<CPC_SCORE_LINEAR>);
+    if (!nu_rect(g))
+        st = g.kind == CPC_SCORE_SOFTPLUS ? launch(nce_umma_bwd_kernel<CPC_SCORE_SOFTPLUS, false>)
+                                          : launch(nce_umma_bwd_kernel<CPC_SCORE_LINEAR, false>);
+    else
+        st = g.kind == CPC_SCORE_SOFTPLUS ? launch(nce_umma_bwd_kernel<CPC_SCORE_SOFTPLUS, true>)
+                                          : launch(nce_umma_bwd_kernel<CPC_SCORE_LINEAR, true>);
     if (st != CPC_OK) return st;
     CPC_LAUNCH_CHECK();
     count_launch(4);

@@ -307,6 +307,27 @@ int cpc_infonce_bwd(const float* pred, const float* targets, const float* lse, c
                     float* d_pred, float* d_targets, const cpc_infonce_params* p,
                     void* workspace, size_t workspace_bytes, void* stream);
 
+/* Rectangular problem: the shard of one data-parallel rank scored against the predictions of the whole global batch
+ * (what nn.DataParallel computes on its gathered outputs).  pred is (pred_batch, K, E) -- the all-gathered predictions --
+ * and targets holds this rank's `batch` items; the positive of local target t is prediction target_offset + t.  The loss
+ * is the reference's block applied to that column block of the global score tensor: logsumexp over all pred_batch (x K)
+ * predictions, mean over the batch (x K) target columns, regulariser mean over the block's entries, max / mean score over
+ * the block.  For W equal shards with target_offset = r * batch, the mean of the W shard losses is the global loss and the
+ * sum of their d_pred is W times the global gradient.
+ * shard == NULL or {batch, 0}: the square problem of the plain entry points (which call these with NULL).  pred_batch <
+ * batch, target_offset outside [0, pred_batch - batch], and any shard for validation (which = 2) are rejected
+ * (CPC_ERR_BAD_SHAPE, workspace size 0) before the device is touched.  d_pred has the shape of pred. */
+typedef struct cpc_infonce_shard {
+    int32_t pred_batch;
+    int32_t target_offset;
+} cpc_infonce_shard;
+size_t cpc_infonce_workspace_bytes_ex(const cpc_infonce_params* p, const cpc_infonce_shard* shard, int which);
+int cpc_infonce_fwd_ex(const float* pred, const float* targets, float* out, float* lse, const cpc_infonce_params* p,
+                       const cpc_infonce_shard* shard, void* workspace, size_t workspace_bytes, void* stream);
+int cpc_infonce_bwd_ex(const float* pred, const float* targets, const float* lse, const float* grad_loss,
+                       float* d_pred, float* d_targets, const cpc_infonce_params* p, const cpc_infonce_shard* shard,
+                       void* workspace, size_t workspace_bytes, void* stream);
+
 /* Validation metrics of ContrastiveEstimationTrainer.validate (contrastive_estimation_training.py:224-247):
  * per-step losses (K) with the reference's view semantics, per-step accuracy (K), mean score (1).
  * metrics: (2*K + 1) fp32. */
