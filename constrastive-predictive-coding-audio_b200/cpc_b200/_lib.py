@@ -121,6 +121,11 @@ SIGNATURES = {
                                           ctypes.c_size_t, _P]),
     "cpc_infonce_bwd_ex": (ctypes.c_int, [_P, _P, _P, _P, _P, _P, ctypes.POINTER(InfoNceParams),
                                           ctypes.POINTER(InfoNceShard), _P, ctypes.c_size_t, _P]),
+    "cpc_infonce_validate_partial_bytes": (ctypes.c_size_t, [ctypes.POINTER(InfoNceParams), ctypes.POINTER(InfoNceShard)]),
+    "cpc_infonce_validate_ex": (ctypes.c_int, [_P, _P, _P, ctypes.POINTER(InfoNceParams), ctypes.POINTER(InfoNceShard), _P,
+                                               ctypes.c_size_t, _P]),
+    "cpc_infonce_validate_combine": (ctypes.c_int, [_P, ctypes.c_int, _P, ctypes.POINTER(InfoNceParams),
+                                                    ctypes.POINTER(InfoNceShard), _P]),
     "cpc_adam_step": (ctypes.c_int, [ctypes.c_int32, _P, _P, _P, _P, _P, _P, ctypes.POINTER(AdamParams), _P]),
 }
 

@@ -1018,6 +1018,74 @@ def infonce_validate(pred, targets, all_steps, kind="linear", precision=None):
     return metrics[:k], metrics[k:2 * k], metrics[2 * k]
 
 
+def infonce_validate_shard(pred_all, targets, all_steps, kind="linear", target_offset=0, precision=None):
+    """One data-parallel rank's share of ``infonce_validate`` on a global batch: pred_all (W*b,K,E) the gathered
+    predictions of every rank in rank order, targets this rank's (b,E,K), ``target_offset = r*b``.  Returns the rank's
+    partial record (a uint8 device tensor of fixed size, layout in cpc_b200.h); ``infonce_validate_combine`` turns the
+    W records, gathered in rank order, into the metrics of ``infonce_validate(cat(pred), cat(targets))``.  With
+    pred_all and targets of the same items (W = 1) the record is the square problem's."""
+    _require_cuda(pred_all, targets)
+    lib = _lib.load()
+    if pred_all.dtype != torch.float32 or targets.dtype != torch.float32:
+        raise _lib.CpcError("infonce_validate_shard expects fp32 tensors")
+    _, k, e = pred_all.shape
+    b = targets.shape[0]
+    if tuple(targets.shape) != (b, e, k):
+        raise ValueError("targets must be (B, E, K) = %s, got %s" % ((b, e, k), tuple(targets.shape)))
+    pred_all = pred_all.detach().contiguous()
+    targets = targets.detach()
+    p = _nce_params(pred_all, targets, all_steps, kind, 0.0, precision or _default_precision)
+    sh = _nce_shard(pred_all, targets, target_offset)
+    shp = ctypes.byref(sh) if sh is not None else None
+    nbytes = lib.cpc_infonce_validate_partial_bytes(ctypes.byref(p), shp)
+    if nbytes == 0:
+        raise ValueError("pred_all of %d items, %d targets at offset %d is not one of W equal rank blocks"
+                         % (pred_all.shape[0], b, target_offset))
+    record = torch.empty(int(nbytes), dtype=torch.uint8, device=pred_all.device)
+    ws = _workspace(lib.cpc_infonce_workspace_bytes_ex(ctypes.byref(p), shp, 2), pred_all.device)
+    with torch.cuda.device(pred_all.device):
+        _call(_nce_key("cpc_infonce_validate_ex", p, sh), _nce_flops(p, sh), lib.cpc_infonce_validate_ex, _ptr(pred_all),
+              _ptr(targets), _ptr(record), ctypes.byref(p), shp, _ptr(ws), ws.numel(), _stream())
+    return record
+
+
+def _nce_combine_args(records, batch, steps, all_steps):
+    """(params, shard or None) of the combine of W = records.shape[0] records of ``batch`` targets each.  The combine
+    reads batch, steps and all_steps; enc and score_kind only have to be valid."""
+    world = records.shape[0]
+    p = _lib.InfoNceParams()
+    p.batch, p.steps, p.enc, p.all_steps, p.score_kind = int(batch), int(steps), 1, int(bool(all_steps)), _lib.SCORE_LINEAR
+    if world == 1:
+        return p, None
+    sh = _lib.InfoNceShard()
+    sh.pred_batch, sh.target_offset = world * int(batch), 0
+    return p, sh
+
+
+def infonce_validate_combine(records, batch, steps, all_steps):
+    """records (W, nbytes) uint8: the ``infonce_validate_shard`` records of W ranks with ``batch`` targets each, in rank
+    order (one all-gather) -> (per_step_losses (K), per_step_accuracy (K), mean_score ()) of the whole W*batch batch,
+    as ``infonce_validate`` returns them.  Deterministic: equal records give bit-identical metrics on every rank."""
+    _require_cuda(records)
+    lib = _lib.load()
+    if records.dtype != torch.uint8 or records.dim() != 2:
+        raise ValueError("records must be a (W, nbytes) uint8 tensor, got %s %s" % (records.dtype, tuple(records.shape)))
+    p, sh = _nce_combine_args(records, batch, steps, all_steps)
+    shp = ctypes.byref(sh) if sh is not None else None
+    if records.shape[1] != lib.cpc_infonce_validate_partial_bytes(ctypes.byref(p), shp):
+        raise ValueError("records of %d bytes do not belong to %d ranks of %d targets, K = %d"
+                         % (records.shape[1], records.shape[0], batch, steps))
+    records = records.contiguous()
+    k = int(steps)
+    metrics = torch.empty(2 * k + 1, dtype=torch.float32, device=records.device)
+    with torch.cuda.device(records.device):
+        _call("cpc_infonce_validate_combine w%d b%d k%d %s" % (records.shape[0], batch, k,
+                                                              "all-steps" if all_steps else "per-step"),
+              0.0, lib.cpc_infonce_validate_combine, _ptr(records), records.shape[0], _ptr(metrics), ctypes.byref(p), shp,
+              _stream(), nbytes=float(records.numel()))
+    return metrics[:k], metrics[k:2 * k], metrics[2 * k]
+
+
 # --------------------------------------------------------------------------------------------------
 # CQT front end (no autograd: the filterbank is frozen in training, constant_q_transform.py:145)
 # --------------------------------------------------------------------------------------------------

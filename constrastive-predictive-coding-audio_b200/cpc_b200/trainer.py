@@ -65,8 +65,9 @@ class ContrastiveEstimationTrainer:
                  prediction_steps=16, verbose=True, global_negatives=False):
         """``global_negatives``: with more than one rank, score each rank's targets against the predictions of every
         rank (the reference's nn.DataParallel objective) instead of its own only; the returned loss and max score are
-        then the global ones on every rank.  Needs a fused score function and no gradient penalty.  validate() keeps
-        per-rank negatives.  No effect on a single rank."""
+        then the global ones on every rank.  Needs a fused score function and no gradient penalty.  validate() scores
+        the whole validation batch with either setting (its ``shard_over_ranks`` splits that work over the ranks).  No
+        effect on a single rank."""
         if global_negatives and score_function not in _FUSED_KINDS:
             raise ValueError("global_negatives needs linear_score_function, softplus_score_function or "
                              "difference_score_function (the fused kernels)")
@@ -229,10 +230,19 @@ class ContrastiveEstimationTrainer:
                 reducer.remove()
 
     # -- validation: fused metrics kernel for the known score functions, literal block otherwise --------
-    def validate(self, batch_size=64, num_workers=1, max_steps=None):
+    def validate(self, batch_size=64, num_workers=1, max_steps=None, shard_over_ranks=False):
+        """Per-step losses, accuracies, mean score and mutual-information bound over the seeded validation batches.
+
+        ``shard_over_ranks`` (with more than one rank): every rank forwards only its contiguous shard of each batch,
+        with rank 0's BatchNorm buffers, and the fused metrics of the whole batch are assembled from one all-gather of
+        the predictions and one of each rank's fixed-size partial record.  Every rank returns the same values, those of
+        rank 0 validating alone, for 1/W of the forward work.  All ranks must call it together.  Needs a fused score
+        function, CUDA and a batch_size the world size divides.  No effect on a single rank."""
         if self.validation_set is None:
             print("No validation set")
             return 0, 0
+        if shard_over_ranks and self.world > 1:
+            return self._validate_sharded(batch_size, num_workers, max_steps)
         self.model.eval()
         sampler = FileBatchSampler(index_count_per_file=self.validation_set.get_example_count_per_file(),
                                    batch_size=batch_size, file_batch_size=8, drop_last=True, seed=0)
@@ -282,6 +292,69 @@ class ContrastiveEstimationTrainer:
         total_losses /= max_steps
         total_accurate /= max_steps
         total_score /= max_steps
+        mutual_information_lb = math.log(n) - total_losses
+        self.model.train()
+        return total_losses, total_accurate, total_score, mutual_information_lb
+
+    def _validate_sharded(self, batch_size, num_workers, max_steps):
+        """validate(shard_over_ranks=True) with W > 1 ranks.  Rank r scores its targets against the gathered
+        predictions (ops.infonce_validate_shard); the W partial records combine into the whole batch's metrics."""
+        kind = _FUSED_KINDS.get(self.score_function)
+        # refused on every rank alike, before any collective
+        if batch_size % self.world:
+            raise ValueError("validation batch_size %d is not divisible by world size %d" % (batch_size, self.world))
+        if kind is None:
+            raise ValueError("validate(shard_over_ranks=True) needs linear_score_function, softplus_score_function or "
+                             "difference_score_function (the fused kernels)")
+        if self.device is None or torch.device(self.device).type != "cuda":
+            raise ValueError("validate(shard_over_ranks=True) runs on CUDA devices only, got device %r" % (self.device,))
+        rank, world, k = self.rank, self.world, self.prediction_steps
+        per = batch_size // world
+        self.model.eval()
+        sampler = FileBatchSampler(index_count_per_file=self.validation_set.get_example_count_per_file(),
+                                   batch_size=batch_size, file_batch_size=8, drop_last=True, seed=0)
+        loader = torch.utils.data.DataLoader(self.validation_set, batch_sampler=sampler, num_workers=num_workers,
+                                             pin_memory=False)
+        total_losses = torch.zeros(k, device=self.device)
+        total_accurate = torch.zeros(k, device=self.device)
+        total_score = torch.zeros((), device=self.device)
+        n = batch_size * k if self.score_over_all_timesteps else batch_size
+        max_steps = len(loader) if max_steps is None else min(max_steps, len(loader))
+        # the reference evaluates replica 0 of nn.DataParallel: rank 0's buffers (BatchNorm running statistics), swapped
+        # in for the loop and this rank's own restored afterwards
+        buffers = list(self.model.buffers())
+        own = [b.detach().clone() for b in buffers]
+        try:
+            with torch.no_grad():
+                for b in buffers:
+                    torch.distributed.broadcast(b, src=0)
+                for step, batch in enumerate(iter(loader)):
+                    batch = batch[rank * per:(rank + 1) * per].to(device=self.device).unsqueeze(1)
+                    if self.preprocessing is not None:
+                        batch = self.preprocessing(batch)
+                    predicted_z, targets, _, _ = self.model(batch)
+                    predicted_z = predicted_z.contiguous()
+                    pred_all = predicted_z.new_empty((world * per,) + tuple(predicted_z.shape[1:]))
+                    torch.distributed.all_gather_into_tensor(pred_all, predicted_z)
+                    record = ops.infonce_validate_shard(pred_all, targets, self.score_over_all_timesteps, kind,
+                                                        target_offset=rank * per)
+                    records = record.new_empty((world, record.numel()))
+                    torch.distributed.all_gather_into_tensor(records, record)
+                    losses, accuracy, mean_score = ops.infonce_validate_combine(records, per, k,
+                                                                                self.score_over_all_timesteps)
+                    total_losses += losses
+                    total_accurate += accuracy
+                    total_score += mean_score
+                    if step + 1 >= max_steps:
+                        break
+        finally:
+            with torch.no_grad():
+                for b, o in zip(buffers, own):
+                    b.copy_(o)
+        del loader
+        total_losses /= max_steps
+        total_accurate /= max_steps
+        total_score = total_score.item() / max_steps                # the one host read of the loop's results
         mutual_information_lb = math.log(n) - total_losses
         self.model.train()
         return total_losses, total_accurate, total_score, mutual_information_lb

@@ -377,6 +377,99 @@ __global__ void __launch_bounds__(256) nce_validate_final_kernel(const float* __
     if (threadIdx.x == 0) metrics[2 * g.K] = out4[3];
 }
 
+// Validation of a data-parallel rank (cpc_infonce_validate_ex): the rank's targets against the gathered predictions
+// of all ranks.  Its partial record (fp32 words, layout in cpc_b200.h):
+//   [0, K)      noise sums: lse of this rank's columns, into the slot the square kernel above gives them
+//   [K, 2K)     valid sums: the positives' scores of this rank's columns, into their slots
+//   [2K]        sum of this rank's scores
+//   [H, H + N)  per gathered prediction row (problem-major, N = nprob * R): best score over this rank's columns
+//   [H + N, H + 2N)  its GLOBAL column index (int32), -1 when no score beats -inf
+// with H = nce_record_header(K).  Slots: all-steps mode, column f = t*K + k' -> k' (local and global f differ by
+// target_offset * K); per-step mode, the lse of (k, t) sits at global flat index k*Bp + t of the reference's
+// re-viewed array and goes to slot (k*Bp + t) mod K, while S_c[b, b] goes to slot c.
+__host__ __device__ __forceinline__ int nce_record_header(int K) { return (2 * K + 1 + 3) / 4 * 4; }
+
+__global__ void __launch_bounds__(256) nce_validate_partial_kernel(const float* __restrict__ lse,
+                                                                  const float* __restrict__ diag,
+                                                                  const float* __restrict__ rowp_m,
+                                                                  const int* __restrict__ rowp_i, int ncoltiles,
+                                                                  const float* __restrict__ cta, int ncta, NceGeom g,
+                                                                  float* __restrict__ rec) {
+    __shared__ float acc_noise[TILE], acc_valid[TILE];
+    __shared__ float red[8];
+    for (int k = threadIdx.x; k < g.K; k += blockDim.x) { acc_noise[k] = 0.f; acc_valid[k] = 0.f; }
+    __syncthreads();
+    for (int f = threadIdx.x; f < g.ncols; f += blockDim.x) {
+        if (g.all) {
+            const int kk = f % g.K;
+            atomicAdd(&acc_noise[kk], lse[f]);
+            atomicAdd(&acc_valid[kk], diag[f]);
+        } else {                                                   // f = prob * C + c, global target t = c + doff
+            const int prob = f / g.C, c = f - prob * g.C;
+            atomicAdd(&acc_noise[(prob * g.Bp + c + g.doff) % g.K], lse[f]);
+            atomicAdd(&acc_valid[prob], diag[f]);
+        }
+    }
+    float sm = 0.f;
+    for (int i = threadIdx.x; i < ncta; i += blockDim.x) sm += cta[i * 3 + 1];
+    sm = block_sum(sm, red);
+    const int H = nce_record_header(g.K), nrows = g.nprob * g.R;
+    float* best_out = rec + H;
+    int* arg_out = reinterpret_cast<int*>(rec + H + nrows);
+    for (int idx = threadIdx.x; idx < nrows; idx += blockDim.x) {
+        const int prob = idx / g.R, r = idx - prob * g.R;
+        float best = -INFINITY;
+        int arg = -1;
+        for (int t = 0; t < ncoltiles; ++t) {                      // column tiles in order: the first maximum wins
+            const size_t o = ((size_t)t * g.nprob + prob) * g.R + r;
+            const float v = rowp_m[o];
+            if (v > best) { best = v; arg = rowp_i[o] + g.doff; }
+        }
+        best_out[idx] = best;
+        arg_out[idx] = arg;
+    }
+    __syncthreads();
+    for (int k = threadIdx.x; k < g.K; k += blockDim.x) { rec[k] = acc_noise[k]; rec[g.K + k] = acc_valid[k]; }
+    if (threadIdx.x == 0)                                          // block_sum's result lives in thread 0
+        for (int i = 2 * g.K; i < H; ++i) rec[i] = i == 2 * g.K ? sm : 0.f;
+}
+
+// The W records of one validation batch, gathered in rank order (rank r's columns are the global block r), -> the
+// metrics of cpc_infonce_validate on the whole batch.  Rank order is column order, so a strict > over the ranks keeps
+// the first maximum.  Sums over the ranks run in rank order: every rank computes bit-identical metrics.
+__global__ void __launch_bounds__(256) nce_validate_combine_kernel(const float* __restrict__ recs, int world, NceGeom g,
+                                                                  float* __restrict__ metrics) {
+    __shared__ int hits[TILE];
+    const int H = nce_record_header(g.K), nrows = g.nprob * g.R;
+    const size_t stride = (size_t)H + 2 * (size_t)nrows;           // words per record
+    for (int k = threadIdx.x; k < g.K; k += blockDim.x) hits[k] = 0;
+    __syncthreads();
+    for (int idx = threadIdx.x; idx < nrows; idx += blockDim.x) {
+        const int prob = idx / g.R, r = idx - prob * g.R;
+        float best = -INFINITY;
+        int arg = -1;
+        for (int w = 0; w < world; ++w) {
+            const float* rec = recs + (size_t)w * stride;
+            const float v = rec[H + idx];
+            if (v > best) { best = v; arg = reinterpret_cast<const int*>(rec + H + nrows)[idx]; }
+        }
+        if (arg == r) atomicAdd(&hits[g.all ? r % g.K : prob], 1);
+    }
+    __syncthreads();
+    const float n = g.all ? (float)g.Bp * (float)g.K : (float)g.Bp;
+    for (int k = threadIdx.x; k < g.K; k += blockDim.x) {
+        double noise = 0.0, valid = 0.0;
+        for (int w = 0; w < world; ++w) { noise += recs[(size_t)w * stride + k]; valid += recs[(size_t)w * stride + g.K + k]; }
+        metrics[k] = (float)(noise - valid) / (float)g.Bp;
+        metrics[g.K + k] = (float)hits[k] / n;
+    }
+    if (threadIdx.x == 0) {
+        double sm = 0.0;
+        for (int w = 0; w < world; ++w) sm += recs[(size_t)w * stride + 2 * g.K];
+        metrics[2 * g.K] = (float)(sm / ((double)g.nprob * g.R * g.R));   // scores of the whole batch's square
+    }
+}
+
 // ---- backward -----------------------------------------------------------------------------------
 // Per-step regulariser, pass 1: rsum[d, t] += S_k[d, t] for every step k (grid (col tiles, row tiles, K); rsum zeroed).
 template <bool kDiff>
@@ -574,6 +667,50 @@ static NceWs nce_ws(const NceGeom& g, void* base) {
     return w;
 }
 
+// Validation shards describe one of W >= 2 equal rank blocks: pred_batch = W * batch, target_offset = r * batch.  The
+// one-rank problem is shard == NULL ({batch, 0} is not a validation shard).
+static int nce_validate_rank_shard(const cpc_infonce_params* p, const cpc_infonce_shard* shard, cpc_infonce_shard* out) {
+    const int st = nce_validate_shard(p, shard, out);
+    if (st != CPC_OK || !shard) return st;
+    if (shard->pred_batch == p->batch || shard->pred_batch % p->batch || shard->target_offset % p->batch)
+        return CPC_ERR_BAD_SHAPE;
+    return CPC_OK;
+}
+
+// Validation workspace behind the forward scratch: lse, 4 scalars, per-(column tile, row) arg-max partials
+struct NceValWs {
+    NceWs w;
+    float *lse, *out4, *rowp_m;
+    int* rowp_i;
+    int ncoltiles;
+};
+static NceValWs nce_val_ws(const NceGeom& g, void* base) {
+    NceValWs v;
+    v.w = nce_ws(g, base);
+    char* b = reinterpret_cast<char*>(base) + v.w.bytes;
+    v.lse = reinterpret_cast<float*>(b);
+    b += align_up(sizeof(float) * (size_t)g.ncols, 256);
+    v.out4 = reinterpret_cast<float*>(b);
+    b += 256;
+    v.ncoltiles = ceil_div(g.C, TILE);
+    const size_t rows = (size_t)v.ncoltiles * g.nprob * g.R;
+    v.rowp_m = reinterpret_cast<float*>(b);
+    v.rowp_i = reinterpret_cast<int*>(b + align_up(sizeof(float) * rows, 256));
+    return v;
+}
+
+// Forward over the (rectangular) validation problem: column statistics -> lse, arg-max partials per column tile.
+static int nce_validate_forward(const float* pred, const float* targets, const NceGeom& g, const NceValWs& v,
+                                cudaStream_t s) {
+    dim3 grid(v.ncoltiles, g.nrowtiles, g.nprob);
+    nce_fwd_launcher(g)<<<grid, TILE_THREADS, 0, s>>>(pred, targets, g, v.w.part_m, v.w.part_s, v.w.diag, v.w.cta,
+                                                      v.rowp_m, v.rowp_i, nullptr);
+    CPC_LAUNCH_CHECK();
+    nce_combine_kernel<<<v.w.nblk, 256, 0, s>>>(v.w.part_m, v.w.part_s, v.w.diag, v.lse, v.w.blk, g.ncols, g.nrowtiles);
+    CPC_LAUNCH_CHECK();
+    return CPC_OK;
+}
+
 }  // namespace cpc
 
 using namespace cpc;
@@ -582,7 +719,7 @@ using namespace cpc;
 extern "C" size_t cpc_infonce_workspace_bytes_ex(const cpc_infonce_params* p, const cpc_infonce_shard* shard, int which) {
     cpc_infonce_shard sh;
     if (nce_validate(p) != CPC_OK || nce_validate_shard(p, shard, &sh) != CPC_OK) return 0;
-    if (which == 2 && shard) return 0;                         // validation keeps per-rank negatives: no shard
+    if (which == 2 && nce_validate_rank_shard(p, shard, &sh) != CPC_OK) return 0;
     const NceGeom g = nce_geom(p, sh);
     if (which == 1)
         return nce_umma_eligible(p, sh, 1) ? nce_umma_workspace(p, sh, 1) : align_up(sizeof(float) * nce_rsum_floats(g), 256);
@@ -686,27 +823,59 @@ extern "C" int cpc_infonce_validate(const float* pred, const float* targets, flo
     if ((st = check_device()) != CPC_OK) return st;
     NceGeom g = nce_geom(p, cpc_infonce_shard{p->batch, 0});
     g.lambda = 0.f;                                            // validation reports the un-regularised loss
-    NceWs w = nce_ws(g, workspace);
-    char* base = reinterpret_cast<char*>(workspace) + w.bytes;
-    float* lse = reinterpret_cast<float*>(base);
-    base += align_up(sizeof(float) * (size_t)g.ncols, 256);
-    float* out4 = reinterpret_cast<float*>(base);
-    base += 256;
-    const int ncoltiles = ceil_div(g.C, TILE);
-    const size_t rows = (size_t)ncoltiles * g.nprob * g.R;
-    float* rowp_m = reinterpret_cast<float*>(base);
-    int* rowp_i = reinterpret_cast<int*>(base + align_up(sizeof(float) * rows, 256));
+    const NceValWs v = nce_val_ws(g, workspace);
     cudaStream_t s = (cudaStream_t)stream;
-    dim3 grid(ncoltiles, g.nrowtiles, g.nprob);
-    nce_fwd_launcher(g)<<<grid, TILE_THREADS, 0, s>>>(pred, targets, g, w.part_m, w.part_s, w.diag, w.cta, rowp_m, rowp_i,
-                                                      nullptr);
+    if ((st = nce_validate_forward(pred, targets, g, v, s)) != CPC_OK) return st;
+    nce_final_kernel<<<1, 256, 0, s>>>(v.w.blk, v.w.nblk, v.w.cta, v.w.ncta, g, v.out4, nullptr);
     CPC_LAUNCH_CHECK();
-    nce_combine_kernel<<<w.nblk, 256, 0, s>>>(w.part_m, w.part_s, w.diag, lse, w.blk, g.ncols, g.nrowtiles);
-    CPC_LAUNCH_CHECK();
-    nce_final_kernel<<<1, 256, 0, s>>>(w.blk, w.nblk, w.cta, w.ncta, g, out4, nullptr);
-    CPC_LAUNCH_CHECK();
-    nce_validate_final_kernel<<<1, 256, 0, s>>>(lse, w.diag, rowp_m, rowp_i, ncoltiles, out4, g, metrics);
+    nce_validate_final_kernel<<<1, 256, 0, s>>>(v.lse, v.w.diag, v.rowp_m, v.rowp_i, v.ncoltiles, v.out4, g, metrics);
     CPC_LAUNCH_CHECK();
     count_launch(4);
+    return CPC_OK;
+}
+
+extern "C" size_t cpc_infonce_validate_partial_bytes(const cpc_infonce_params* p, const cpc_infonce_shard* shard) {
+    cpc_infonce_shard sh;
+    if (nce_validate(p) != CPC_OK || nce_validate_rank_shard(p, shard, &sh) != CPC_OK) return 0;
+    const NceGeom g = nce_geom(p, sh);
+    return sizeof(float) * ((size_t)nce_record_header(g.K) + 2 * (size_t)g.nprob * g.R);
+}
+
+extern "C" int cpc_infonce_validate_ex(const float* pred, const float* targets, void* partial,
+                                       const cpc_infonce_params* p, const cpc_infonce_shard* shard, void* workspace,
+                                       size_t workspace_bytes, void* stream) {
+    int st = nce_validate(p);
+    if (st != CPC_OK) return st;
+    cpc_infonce_shard sh;
+    if ((st = nce_validate_rank_shard(p, shard, &sh)) != CPC_OK) return st;
+    if (!pred || !targets || !partial) return CPC_ERR_NULL;
+    if (!workspace || workspace_bytes < cpc_infonce_workspace_bytes_ex(p, shard, 2)) return CPC_ERR_WORKSPACE;
+    if ((st = check_device()) != CPC_OK) return st;
+    NceGeom g = nce_geom(p, sh);
+    g.lambda = 0.f;
+    const NceValWs v = nce_val_ws(g, workspace);
+    cudaStream_t s = (cudaStream_t)stream;
+    if ((st = nce_validate_forward(pred, targets, g, v, s)) != CPC_OK) return st;
+    nce_validate_partial_kernel<<<1, 256, 0, s>>>(v.lse, v.w.diag, v.rowp_m, v.rowp_i, v.ncoltiles, v.w.cta, v.w.ncta, g,
+                                                  reinterpret_cast<float*>(partial));
+    CPC_LAUNCH_CHECK();
+    count_launch(3);
+    return CPC_OK;
+}
+
+extern "C" int cpc_infonce_validate_combine(const void* partials, int world, float* metrics,
+                                            const cpc_infonce_params* p, const cpc_infonce_shard* shard, void* stream) {
+    int st = nce_validate(p);
+    if (st != CPC_OK) return st;
+    cpc_infonce_shard sh;
+    if ((st = nce_validate_rank_shard(p, shard, &sh)) != CPC_OK) return st;
+    if (world < 1 || (int64_t)world * p->batch != sh.pred_batch) return CPC_ERR_BAD_SHAPE;
+    if (!partials || !metrics) return CPC_ERR_NULL;
+    if ((st = check_device()) != CPC_OK) return st;
+    const NceGeom g = nce_geom(p, sh);
+    nce_validate_combine_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(reinterpret_cast<const float*>(partials), world, g,
+                                                                    metrics);
+    CPC_LAUNCH_CHECK();
+    count_launch();
     return CPC_OK;
 }

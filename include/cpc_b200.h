@@ -315,8 +315,9 @@ int cpc_infonce_bwd(const float* pred, const float* targets, const float* lse, c
  * the block.  For W equal shards with target_offset = r * batch, the mean of the W shard losses is the global loss and the
  * sum of their d_pred is W times the global gradient.
  * shard == NULL or {batch, 0}: the square problem of the plain entry points (which call these with NULL).  pred_batch <
- * batch, target_offset outside [0, pred_batch - batch], and any shard for validation (which = 2) are rejected
- * (CPC_ERR_BAD_SHAPE, workspace size 0) before the device is touched.  d_pred has the shape of pred. */
+ * batch and target_offset outside [0, pred_batch - batch] are rejected (CPC_ERR_BAD_SHAPE, workspace size 0) before the
+ * device is touched; so are validation shards (which = 2) that are not one of W >= 2 equal rank blocks (see
+ * cpc_infonce_validate_ex).  d_pred has the shape of pred. */
 typedef struct cpc_infonce_shard {
     int32_t pred_batch;
     int32_t target_offset;
@@ -333,6 +334,30 @@ int cpc_infonce_bwd_ex(const float* pred, const float* targets, const float* lse
  * metrics: (2*K + 1) fp32. */
 int cpc_infonce_validate(const float* pred, const float* targets, float* metrics,
                          const cpc_infonce_params* p, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Validation sharded over W data-parallel ranks: the metrics of cpc_infonce_validate on the whole batch of B_g = W*batch
+ * items, each rank scoring only its own targets.  Rank r passes the gathered predictions (B_g, K, E) in rank order, its
+ * targets and shard {pred_batch = W*batch, target_offset = r*batch}, W >= 2 (shard == NULL: the one-rank record of the
+ * square problem).  cpc_infonce_validate_ex writes the rank's partial record (partial_bytes, device memory; workspace:
+ * cpc_infonce_workspace_bytes_ex(p, shard, 2)); cpc_infonce_validate_combine reads the W records concatenated in rank
+ * order and writes the (2*K + 1) metrics; every rank that combines the same records gets bit-identical metrics.
+ * p->regularization is ignored, as in cpc_infonce_validate; the combine reads batch, steps and all_steps of p (which
+ * must pass the same checks) and shard->pred_batch, which must equal world * batch.  Record, in 4-byte words, with
+ * H = 2*K + 1 rounded up to a multiple of 4 and N = B_g*K gathered prediction rows (all-steps: rows (d, k); per-step:
+ * problem-major, K x B_g rows d):
+ *   [0, K)   sum of lse over this rank's softmax columns, by per-step loss slot (all-steps: column (t, k') -> slot k';
+ *            per-step: the lse of (k, t) -> slot (k*B_g + t) mod K, the reference's re-viewed noise array)
+ *   [K, 2K)  sum of the positives' scores of this rank's columns, by slot (k' resp. the problem k)
+ *   [2K]     sum of this rank's scores; up to H: zero
+ *   [H, H+N) fp32 best score of each row over this rank's columns; [H+N, H+2N) int32 its global column index
+ *            (first maximum; -1 if no score beats -inf).
+ * Bad or non-rank shards, world < 1, world*batch != pred_batch, NULL pointers and a short workspace are rejected before
+ * the device is touched (partial_bytes 0). */
+size_t cpc_infonce_validate_partial_bytes(const cpc_infonce_params* p, const cpc_infonce_shard* shard);
+int cpc_infonce_validate_ex(const float* pred, const float* targets, void* partial, const cpc_infonce_params* p,
+                            const cpc_infonce_shard* shard, void* workspace, size_t workspace_bytes, void* stream);
+int cpc_infonce_validate_combine(const void* partials, int world, float* metrics, const cpc_infonce_params* p,
+                                 const cpc_infonce_shard* shard, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * 5. Adam update of all parameter tensors (torch.optim.Adam semantics, amsgrad off) in one pass.
