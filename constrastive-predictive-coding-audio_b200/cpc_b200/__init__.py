@@ -8,6 +8,7 @@ Public surface mirrors the reference's modules (SURVEY.md 8b):
     trainer  : ContrastiveEstimationTrainer, linear/softplus/difference_score_function
     sampler  : FileBatchSampler, SyntheticAudioDataset
     audio_dataset: AudioDataset, AudioTestingDataset (WAV folders as one item stream)
+    device_loader: DeviceBatchLoader (AudioDataset batches decoded and assembled on the GPU from raw PCM bytes)
     ddp      : one-process-per-GPU gradient averaging
     optim    : Adam (torch.optim.Adam semantics, one kernel per step)
     snapshots: state_dict of the reference's whole-model snapshot pickles, without importing reference code

@@ -66,6 +66,16 @@ class InfoNceShard(ctypes.Structure):
     _fields_ = [("pred_batch", ctypes.c_int32), ("target_offset", ctypes.c_int32)]
 
 
+class PcmSegment(ctypes.Structure):
+    _fields_ = [("src_byte_offset", ctypes.c_int64), ("frames", ctypes.c_int32), ("sample_width", ctypes.c_int32),
+                ("block_align", ctypes.c_int32), ("dst_item", ctypes.c_int32), ("dst_offset", ctypes.c_int32)]
+
+
+class PcmParams(ctypes.Structure):
+    _fields_ = [("batch", ctypes.c_int32), ("item_length", ctypes.c_int32), ("out_row_stride", ctypes.c_int64),
+                ("n_segments", ctypes.c_int32)]
+
+
 class AdamParams(ctypes.Structure):
     _fields_ = [("lr", ctypes.c_double), ("beta1", ctypes.c_double), ("beta2", ctypes.c_double), ("eps", ctypes.c_double),
                 ("weight_decay", ctypes.c_double), ("grad_scale", ctypes.c_float), ("maximize", ctypes.c_int32)]
@@ -127,6 +137,7 @@ SIGNATURES = {
     "cpc_infonce_validate_combine": (ctypes.c_int, [_P, ctypes.c_int, _P, ctypes.POINTER(InfoNceParams),
                                                     ctypes.POINTER(InfoNceShard), _P]),
     "cpc_adam_step": (ctypes.c_int, [ctypes.c_int32, _P, _P, _P, _P, _P, _P, ctypes.POINTER(AdamParams), _P]),
+    "cpc_pcm_assemble": (ctypes.c_int, [ctypes.POINTER(PcmParams), _P, _P, _P, _P, _P]),
 }
 
 _lib = None

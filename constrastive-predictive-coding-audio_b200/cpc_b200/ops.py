@@ -6,6 +6,7 @@ libcpc_b200.so.  Every op raises on non-CUDA tensors -- there is no CPU path.
 import contextlib
 import ctypes
 
+import numpy as np
 import torch
 from torch.autograd.function import once_differentiable
 
@@ -1084,6 +1085,52 @@ def infonce_validate_combine(records, batch, steps, all_steps):
               0.0, lib.cpc_infonce_validate_combine, _ptr(records), records.shape[0], _ptr(metrics), ctypes.byref(p), shp,
               _stream(), nbytes=float(records.numel()))
     return metrics[:k], metrics[k:2 * k], metrics[2 * k]
+
+
+# --------------------------------------------------------------------------------------------------
+# PCM batch assembly (the input path of device_loader.DeviceBatchLoader)
+# --------------------------------------------------------------------------------------------------
+
+# numpy mirror of cpc_pcm_segment (32 bytes, the C layout with its tail padding)
+PCM_SEGMENT_DTYPE = np.dtype({"names": ["src_byte_offset", "frames", "sample_width", "block_align", "dst_item",
+                                        "dst_offset"],
+                              "formats": ["<i8", "<i4", "<i4", "<i4", "<i4", "<i4"],
+                              "offsets": [0, 8, 12, 16, 20, 24], "itemsize": ctypes.sizeof(_lib.PcmSegment)})
+
+
+def pcm_assemble(segments, segments_dev, raw_dev, out):
+    """Decode raw PCM frames into the fp32 batch ``out`` (cpc_pcm_assemble), on the current stream.
+
+    ``segments``: the host table, a contiguous numpy array of ``PCM_SEGMENT_DTYPE`` (validated by the library);
+    ``segments_dev``: the same bytes in device memory (uint8, 8-byte aligned); ``raw_dev``: uint8 device tensor that
+    the segments' byte offsets index; ``out``: (B, L) fp32 on the device with unit column stride -- rows may be strided
+    (a column slice of a wider tensor such as ``GraphedTrainStep.static_batch``), columns past L are left untouched."""
+    _require_cuda(segments_dev, raw_dev, out)
+    lib = _lib.load()
+    if out.dtype != torch.float32 or out.dim() != 2 or out.stride(1) != 1:
+        raise ValueError("out must be a (B, L) float32 tensor with unit column stride, got %s %s stride %s"
+                         % (out.dtype, tuple(out.shape), out.stride()))
+    segments = np.ascontiguousarray(segments)
+    if segments.dtype != PCM_SEGMENT_DTYPE or segments.ndim != 1:
+        raise ValueError("segments must be a 1-d array of ops.PCM_SEGMENT_DTYPE")
+    if segments_dev.dtype != torch.uint8 or segments_dev.numel() < segments.nbytes:
+        raise ValueError("segments_dev must be a uint8 device tensor holding the %d-byte table" % segments.nbytes)
+    if raw_dev.dtype != torch.uint8:
+        raise ValueError("raw_dev must be a uint8 device tensor")
+    if len(segments):
+        live = segments["frames"] > 0
+        end = (segments["src_byte_offset"] + (segments["frames"].astype(np.int64) - 1) * segments["block_align"]
+               + segments["sample_width"])
+        if live.any() and int(end[live].max()) > raw_dev.numel():
+            raise ValueError("a segment reads past the %d raw bytes" % raw_dev.numel())
+    p = _lib.PcmParams()
+    p.batch, p.item_length, p.out_row_stride, p.n_segments = out.shape[0], out.shape[1], out.stride(0), len(segments)
+    read = float((segments["frames"].astype(np.int64) * segments["sample_width"]).sum()) if len(segments) else 0.0
+    with torch.cuda.device(out.device):
+        _call("cpc_pcm_assemble b%d l%d" % (out.shape[0], out.shape[1]), 0.0, lib.cpc_pcm_assemble, ctypes.byref(p),
+              ctypes.c_void_p(segments.ctypes.data), _ptr(segments_dev), _ptr(raw_dev), _ptr(out), _stream(),
+              nbytes=read + 4.0 * out.shape[0] * out.shape[1])
+    return out
 
 
 # --------------------------------------------------------------------------------------------------

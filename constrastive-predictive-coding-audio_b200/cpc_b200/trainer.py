@@ -12,6 +12,7 @@ Multi-GPU: one process per GPU.  Each rank trains on its contiguous slice of eve
 ranks every target against the predictions of the whole global batch, as the reference's nn.DataParallel does
 (``ddp`` module docstring).
 """
+import contextlib
 import math
 import time
 
@@ -20,7 +21,7 @@ import torch.nn.functional as F
 import torch.optim
 import torch.utils.data
 
-from . import ddp, ops, optim
+from . import ddp, device_loader, ops, optim
 from .sampler import FileBatchSampler
 
 
@@ -176,12 +177,22 @@ class ContrastiveEstimationTrainer:
             torch.distributed.all_reduce(flag, op=torch.distributed.ReduceOp.MAX)
         return bool(flag.item())
 
+    def _device_loader(self, dataset, sampler, rank=0, world=1):
+        """``device_loader.DeviceBatchLoader`` for ``dataset``: raises ValueError for a non-CUDA device or a dataset it
+        cannot serve.  Builds nothing that communicates, so callers create it before their first collective."""
+        return device_loader.DeviceBatchLoader(dataset, sampler, self.device, rank=rank, world=world)
+
     def train(self, batch_size=32, epochs=10, lr=0.0001, continue_training_at_step=0, num_workers=1, max_steps=None,
-              profile=False):
+              profile=False, device_loading=False):
+        """``device_loading``: read the batches with ``device_loader.DeviceBatchLoader`` -- raw PCM bytes copied by a
+        host thread, decoded and assembled on the GPU -- instead of a DataLoader over the dataset; the batches are
+        bit-identical, ``num_workers`` is ignored.  Needs a CUDA device and an AudioDataset of integer PCM WAV files
+        (ValueError on every rank otherwise, before any collective)."""
         self.model.train()
         optimizer = self.make_optimizer(lr)
         sampler = FileBatchSampler(index_count_per_file=self.dataset.get_example_count_per_file(),
                                    batch_size=batch_size, file_batch_size=self.file_batch_size, drop_last=True)
+        loader = self._device_loader(self.dataset, sampler, self.rank, self.world) if device_loading else None
         reducer = None
         if self.world > 1:
             # every rank starts from rank 0's weights and sees rank 0's batches: the sampler draws from rank 0's
@@ -190,8 +201,11 @@ class ContrastiveEstimationTrainer:
             ddp.broadcast_parameters(self.model)
             sampler = ddp.ShardedBatchSampler(sampler, self.rank, self.world)
             reducer = ddp.GradientBucketReducer(self.model)
-        dataloader = torch.utils.data.DataLoader(self.dataset, batch_sampler=sampler, num_workers=num_workers,
-                                                 pin_memory=True)
+        if loader is not None:                                   # shards the sampler itself, like the line above
+            dataloader = loader
+        else:
+            dataloader = torch.utils.data.DataLoader(self.dataset, batch_sampler=sampler, num_workers=num_workers,
+                                                     pin_memory=True)
         self.training_step = continue_training_at_step
         try:
             for current_epoch in range(epochs):
@@ -228,26 +242,34 @@ class ContrastiveEstimationTrainer:
         finally:
             if reducer is not None:
                 reducer.remove()
+            if loader is not None:
+                loader.close()
 
     # -- validation: fused metrics kernel for the known score functions, literal block otherwise --------
-    def validate(self, batch_size=64, num_workers=1, max_steps=None, shard_over_ranks=False):
+    def validate(self, batch_size=64, num_workers=1, max_steps=None, shard_over_ranks=False, device_loading=False):
         """Per-step losses, accuracies, mean score and mutual-information bound over the seeded validation batches.
 
         ``shard_over_ranks`` (with more than one rank): every rank forwards only its contiguous shard of each batch,
         with rank 0's BatchNorm buffers, and the fused metrics of the whole batch are assembled from one all-gather of
         the predictions and one of each rank's fixed-size partial record.  Every rank returns the same values, those of
         rank 0 validating alone, for 1/W of the forward work.  All ranks must call it together.  Needs a fused score
-        function, CUDA and a batch_size the world size divides.  No effect on a single rank."""
+        function, CUDA and a batch_size the world size divides.  No effect on a single rank.
+
+        ``device_loading``: read the batches as ``train(device_loading=True)`` does (same values; ``num_workers`` is
+        ignored).  With ``shard_over_ranks`` every rank then reads only its shard of each batch, else the whole batch."""
         if self.validation_set is None:
             print("No validation set")
             return 0, 0
         if shard_over_ranks and self.world > 1:
-            return self._validate_sharded(batch_size, num_workers, max_steps)
-        self.model.eval()
+            return self._validate_sharded(batch_size, num_workers, max_steps, device_loading)
         sampler = FileBatchSampler(index_count_per_file=self.validation_set.get_example_count_per_file(),
                                    batch_size=batch_size, file_batch_size=8, drop_last=True, seed=0)
-        loader = torch.utils.data.DataLoader(self.validation_set, batch_sampler=sampler, num_workers=num_workers,
-                                             pin_memory=False)
+        if device_loading:
+            loader = self._device_loader(self.validation_set, sampler)
+        else:
+            loader = torch.utils.data.DataLoader(self.validation_set, batch_sampler=sampler, num_workers=num_workers,
+                                                 pin_memory=False)
+        self.model.eval()
         k = self.prediction_steps
         total_losses = torch.zeros(k, device=self.device)
         total_accurate = torch.zeros(k, device=self.device)
@@ -256,7 +278,7 @@ class ContrastiveEstimationTrainer:
         template = template.view(batch_size, k) if self.score_over_all_timesteps else template.unsqueeze(1).repeat(1, k)
         total_score = 0
         max_steps = len(loader) if max_steps is None else min(max_steps, len(loader))
-        with torch.no_grad():
+        with torch.no_grad(), (loader if device_loading else contextlib.nullcontext()):
             for step, batch in enumerate(iter(loader)):
                 batch = batch.to(device=self.device).unsqueeze(1)
                 if self.preprocessing is not None:
@@ -296,7 +318,7 @@ class ContrastiveEstimationTrainer:
         self.model.train()
         return total_losses, total_accurate, total_score, mutual_information_lb
 
-    def _validate_sharded(self, batch_size, num_workers, max_steps):
+    def _validate_sharded(self, batch_size, num_workers, max_steps, device_loading=False):
         """validate(shard_over_ranks=True) with W > 1 ranks.  Rank r scores its targets against the gathered
         predictions (ops.infonce_validate_shard); the W partial records combine into the whole batch's metrics."""
         kind = _FUSED_KINDS.get(self.score_function)
@@ -310,11 +332,14 @@ class ContrastiveEstimationTrainer:
             raise ValueError("validate(shard_over_ranks=True) runs on CUDA devices only, got device %r" % (self.device,))
         rank, world, k = self.rank, self.world, self.prediction_steps
         per = batch_size // world
-        self.model.eval()
         sampler = FileBatchSampler(index_count_per_file=self.validation_set.get_example_count_per_file(),
                                    batch_size=batch_size, file_batch_size=8, drop_last=True, seed=0)
-        loader = torch.utils.data.DataLoader(self.validation_set, batch_sampler=sampler, num_workers=num_workers,
-                                             pin_memory=False)
+        if device_loading:                                       # yields this rank's shard of every batch
+            loader = self._device_loader(self.validation_set, sampler, rank, world)
+        else:
+            loader = torch.utils.data.DataLoader(self.validation_set, batch_sampler=sampler, num_workers=num_workers,
+                                                 pin_memory=False)
+        self.model.eval()
         total_losses = torch.zeros(k, device=self.device)
         total_accurate = torch.zeros(k, device=self.device)
         total_score = torch.zeros((), device=self.device)
@@ -329,7 +354,9 @@ class ContrastiveEstimationTrainer:
                 for b in buffers:
                     torch.distributed.broadcast(b, src=0)
                 for step, batch in enumerate(iter(loader)):
-                    batch = batch[rank * per:(rank + 1) * per].to(device=self.device).unsqueeze(1)
+                    if not device_loading:
+                        batch = batch[rank * per:(rank + 1) * per]
+                    batch = batch.to(device=self.device).unsqueeze(1)
                     if self.preprocessing is not None:
                         batch = self.preprocessing(batch)
                     predicted_z, targets, _, _ = self.model(batch)
@@ -348,6 +375,8 @@ class ContrastiveEstimationTrainer:
                     if step + 1 >= max_steps:
                         break
         finally:
+            if device_loading:
+                loader.close()
             with torch.no_grad():
                 for b, o in zip(buffers, own):
                     b.copy_(o)

@@ -381,6 +381,43 @@ int cpc_adam_step(int32_t n_tensors, void* const* params, const void* const* gra
                   void* const* exp_avg_sq, const int64_t* numel, float* step_state,
                   const cpc_adam_params* p, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * 6. Batch assembly from raw PCM WAV bytes (the input path of AudioDataset, audio_dataset.py:61-113).
+ *    The host copies the bytes of whole interleaved frames; one kernel decodes the first channel of each and writes
+ *    the (batch, item_length) fp32 batch, bit-identical to read_wav's numpy conversion:
+ *      width 1: (u8 - 128) / 128    width 2: int16 / 2^15    width 3: sign-extended 24-bit / 2^23
+ *      width 4: int32 rounded to fp32 (nearest even), then / 2^31
+ *    Segment s decodes frames [0, frames) starting at raw + src_byte_offset, frame f at byte src_byte_offset +
+ *    f * block_align (little-endian sample of sample_width bytes, no alignment required), into
+ *    out[dst_item * out_row_stride + dst_offset + f].
+ *    The table is listed item by item (dst_item 0, 1, ..., batch - 1, each at least once) and, within an item, by
+ *    ascending dst_offset; the segments of every item tile [0, item_length) exactly (frames == 0 is allowed and writes
+ *    nothing).  Columns [item_length, out_row_stride) of every row are not touched.
+ *    The table is read twice: segments_host (host memory) is validated and sizes the grid, segments_dev (the same
+ *    bytes in device memory, 8-byte aligned) is what the kernel reads.  Any violation -- width not in 1..4,
+ *    block_align < sample_width, negative counts or offsets, n_segments < 1, out_row_stride < item_length, a segment
+ *    outside [0, item_length) or [0, batch), items out of order, gaps or overlaps -- returns CPC_ERR_BAD_SHAPE, NULL
+ *    pointers CPC_ERR_NULL, a misaligned segments_dev / out CPC_ERR_ALIGNMENT, all before the device is touched.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct cpc_pcm_segment {
+    int64_t src_byte_offset;   /* byte offset of the segment's first frame inside raw                       */
+    int32_t frames;            /* frames to decode                                                          */
+    int32_t sample_width;      /* bytes per sample: 1, 2, 3 or 4                                            */
+    int32_t block_align;       /* bytes per interleaved frame (channels * sample_width); channel 0 is read  */
+    int32_t dst_item;          /* row of out                                                                */
+    int32_t dst_offset;        /* column of the segment's first frame                                       */
+} cpc_pcm_segment;             /* 32 bytes (4 bytes of tail padding)                                        */
+
+typedef struct cpc_pcm_params {
+    int32_t batch;             /* rows of out                                                               */
+    int32_t item_length;       /* L: columns written per row                                                */
+    int64_t out_row_stride;    /* elements between rows of out (>= L)                                       */
+    int32_t n_segments;
+} cpc_pcm_params;
+
+int cpc_pcm_assemble(const cpc_pcm_params* p, const cpc_pcm_segment* segments_host, const cpc_pcm_segment* segments_dev,
+                     const void* raw_dev, float* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
