@@ -137,6 +137,7 @@ SIGNATURES = {
     "cpc_infonce_validate_combine": (ctypes.c_int, [_P, ctypes.c_int, _P, ctypes.POINTER(InfoNceParams),
                                                     ctypes.POINTER(InfoNceShard), _P]),
     "cpc_adam_step": (ctypes.c_int, [ctypes.c_int32, _P, _P, _P, _P, _P, _P, ctypes.POINTER(AdamParams), _P]),
+    "cpc_adam_step_ex": (ctypes.c_int, [ctypes.c_int32, _P, _P, _P, _P, _P, _P, _P, ctypes.POINTER(AdamParams), _P]),
     "cpc_pcm_assemble": (ctypes.c_int, [ctypes.POINTER(PcmParams), _P, _P, _P, _P, _P]),
 }
 

@@ -52,9 +52,12 @@ class Adam(torch.optim.Optimizer):
         return ps, counter
 
     @torch.no_grad()
-    def step(self, closure=None, flat_grads=None, grad_scale=1.0):
+    def step(self, closure=None, flat_grads=None, grad_scale=1.0, skip_if=None):
         """``flat_grads``: optional {param: tensor} overriding ``p.grad`` as the gradient source (the all-reduced
-        flat buffer of the multi-GPU step); ``grad_scale`` multiplies every gradient (1 / world size there)."""
+        flat buffer of the multi-GPU step); ``grad_scale`` multiplies every gradient (1 / world size there).
+        ``skip_if``: optional one-element fp32 tensor on the parameters' device, read by the kernels when they run; a
+        non-zero value leaves parameters, moments and the step count untouched (``cpc_adam_step_ex``), so a step
+        captured in a CUDA graph decides at each replay whether it applies."""
         loss = None
         if closure is not None:
             with torch.enable_grad():
@@ -84,9 +87,17 @@ class Adam(torch.optim.Optimizer):
                                 float(group['eps']), float(group['weight_decay']), float(grad_scale),
                                 int(bool(group['maximize'])))
             numel = float(sum(p.numel() for p in ps))
+            if skip_if is not None and (skip_if.dtype != torch.float32 or skip_if.numel() != 1
+                                        or skip_if.device != ps[0].device):
+                raise _lib.CpcError("cpc_b200.optim.Adam: skip_if must be a one-element fp32 tensor on %s" % ps[0].device)
             with torch.cuda.device(ps[0].device):
-                ops._call("cpc_adam_step n%d" % len(ps), 0.0, lib.cpc_adam_step, len(ps), t[0], t[1], t[2], t[3], t[4],
-                          ops._ptr(counter), ctypes.byref(a), ops._stream(), nbytes=28.0 * numel)
+                if skip_if is None:
+                    ops._call("cpc_adam_step n%d" % len(ps), 0.0, lib.cpc_adam_step, len(ps), t[0], t[1], t[2], t[3],
+                              t[4], ops._ptr(counter), ctypes.byref(a), ops._stream(), nbytes=28.0 * numel)
+                else:
+                    ops._call("cpc_adam_step_ex n%d" % len(ps), 0.0, lib.cpc_adam_step_ex, len(ps), t[0], t[1], t[2],
+                              t[3], t[4], ops._ptr(counter), ops._ptr(skip_if), ctypes.byref(a), ops._stream(),
+                              nbytes=28.0 * numel)
         return loss
 
     def state_dict(self):

@@ -183,13 +183,35 @@ class ContrastiveEstimationTrainer:
         return device_loader.DeviceBatchLoader(dataset, sampler, self.device, rank=rank, world=world)
 
     def train(self, batch_size=32, epochs=10, lr=0.0001, continue_training_at_step=0, num_workers=1, max_steps=None,
-              profile=False, device_loading=False):
+              profile=False, device_loading=False, cuda_graph=False):
         """``device_loading``: read the batches with ``device_loader.DeviceBatchLoader`` -- raw PCM bytes copied by a
         host thread, decoded and assembled on the GPU -- instead of a DataLoader over the dataset; the batches are
         bit-identical, ``num_workers`` is ignored.  Needs a CUDA device and an AudioDataset of integer PCM WAV files
-        (ValueError on every rank otherwise, before any collective)."""
+        (ValueError on every rank otherwise, before any collective).
+
+        ``cuda_graph``: capture the whole step (forward, backward, gradient all-reduce, Adam) into one CUDA graph at the
+        first batch (``GraphedTrainStep(stop_on_nan=True)``, warmed up on that batch) and replay it for every batch of
+        the call; each step is one copy into the graph's input, one replay and one host read of (loss, max score, stop
+        flag).  The NaN stop is decided on the device, over all ranks, before the optimizer runs, so the step at which
+        train() returns and the weights, Adam state and BatchNorm statistics it leaves are those of the eager loop.
+        One difference: after a NaN stop ``.grad`` holds the NaN step's gradients (the eager loop returns before its
+        backward and keeps the previous step's).  Needs a CUDA device and an optimizer that ``make_optimizer`` turns
+        into ``cpc_b200.optim.Adam``; the gradient penalty and ``profile`` are not supported (ValueError on every rank,
+        before any collective)."""
+        if cuda_graph:
+            if self.device is None or torch.device(self.device).type != "cuda":
+                raise ValueError("train(cuda_graph=True) runs on CUDA devices only, got device %r" % (self.device,))
+            if self.wasserstein_gradient_penalty:
+                raise ValueError("train(cuda_graph=True) does not capture the gradient penalty's second-order step")
+            if profile:
+                raise ValueError("train(cuda_graph=True) does not support profile=True: the autograd profiler cannot "
+                                 "see inside a replayed graph")
         self.model.train()
         optimizer = self.make_optimizer(lr)
+        if cuda_graph and not isinstance(optimizer, optim.Adam):
+            raise ValueError("train(cuda_graph=True) needs torch.optim.Adam (run as cpc_b200.optim.Adam) or "
+                             "cpc_b200.optim.Adam on a model whose parameters are all on the GPU; got %s"
+                             % type(optimizer).__name__)
         sampler = FileBatchSampler(index_count_per_file=self.dataset.get_example_count_per_file(),
                                    batch_size=batch_size, file_batch_size=self.file_batch_size, drop_last=True)
         loader = self._device_loader(self.dataset, sampler, self.rank, self.world) if device_loading else None
@@ -200,13 +222,15 @@ class ContrastiveEstimationTrainer:
             # broadcast, and each rank loads only its contiguous shard of every batch (DataParallel.scatter chunking)
             ddp.broadcast_parameters(self.model)
             sampler = ddp.ShardedBatchSampler(sampler, self.rank, self.world)
-            reducer = ddp.GradientBucketReducer(self.model)
+            if not cuda_graph:                                   # the graph reduces its gradients itself
+                reducer = ddp.GradientBucketReducer(self.model)
         if loader is not None:                                   # shards the sampler itself, like the line above
             dataloader = loader
         else:
             dataloader = torch.utils.data.DataLoader(self.dataset, batch_sampler=sampler, num_workers=num_workers,
                                                      pin_memory=True)
         self.training_step = continue_training_at_step
+        graphed = None
         try:
             for current_epoch in range(epochs):
                 if self.verbose:
@@ -214,21 +238,36 @@ class ContrastiveEstimationTrainer:
                 with torch.autograd.profiler.profile(use_device='cuda', enabled=profile) as prof:
                     for batch in iter(dataloader):
                         batch = batch.to(device=self.device, non_blocking=True)
-                        loss, max_score = self.loss_on_batch(batch)
-                        # :124-133 -- the reference leaves BEFORE backward / optimizer.step, so weights and optimizer
-                        # state stay finite
-                        if self._any_rank_nan(loss):
-                            print("nan loss")
-                            print("returned with nan loss at step", self.training_step)
-                            self.last_loss = float("nan")
-                            return
-                        self.model.zero_grad()
-                        loss.backward()
-                        if reducer is not None:
-                            reducer.finish()
-                        optimizer.step()
-                        # one host read per step for (loss, max score)
-                        loss_value, max_value = torch.stack([loss.detach(), max_score.detach()]).tolist()
+                        if cuda_graph:
+                            if graphed is None:                  # every batch has this shape: drop_last=True
+                                graphed = GraphedTrainStep(self, optimizer, tuple(batch.shape), stop_on_nan=True,
+                                                           example_batch=batch)
+                            loss, max_score = graphed(batch)
+                            # one host read per step for (loss, max score, stop flag); the optimizer already skipped
+                            # a NaN step on the device
+                            loss_value, max_value, stopped = torch.cat(
+                                [loss.reshape(1), max_score.reshape(1), graphed.stopped]).tolist()
+                            if stopped:
+                                print("nan loss")
+                                print("returned with nan loss at step", self.training_step)
+                                self.last_loss = float("nan")
+                                return
+                        else:
+                            loss, max_score = self.loss_on_batch(batch)
+                            # :124-133 -- the reference leaves BEFORE backward / optimizer.step, so weights and
+                            # optimizer state stay finite
+                            if self._any_rank_nan(loss):
+                                print("nan loss")
+                                print("returned with nan loss at step", self.training_step)
+                                self.last_loss = float("nan")
+                                return
+                            self.model.zero_grad()
+                            loss.backward()
+                            if reducer is not None:
+                                reducer.finish()
+                            optimizer.step()
+                            # one host read per step for (loss, max score)
+                            loss_value, max_value = torch.stack([loss.detach(), max_score.detach()]).tolist()
                         self.last_loss, self.last_max_score = loss_value, max_value
                         if self.logger is not None:
                             self.logger.loss_meter.update(loss_value)
@@ -242,6 +281,9 @@ class ContrastiveEstimationTrainer:
         finally:
             if reducer is not None:
                 reducer.remove()
+            if graphed is not None:
+                graphed.remove_hooks()
+                graphed = None                                   # drops the graph and its private memory pool
             if loader is not None:
                 loader.close()
 
@@ -406,13 +448,27 @@ class GraphedTrainStep:
     straight from the flat buffer (scaled by 1 / world): no flatten / un-flatten copies.  For e24 the AR model and the
     prediction head (70 % of the bytes) are reduced under the ~8 ms of encoder backward that follow them; only the
     last bucket (the first encoder blocks, < 1 MB) is exposed.  If the NCCL build cannot be captured the step falls back
-    to two graphs around one eager all-reduce (``overlap_description`` says which)."""
+    to two graphs around one eager all-reduce (``overlap_description`` says which).
 
-    def __init__(self, trainer, optimizer, batch_shape, warmup=3, bucket_mb=12.0):
+    ``stop_on_nan=True`` (needs ``cpc_b200.optim.Adam``) keeps the reference's NaN stop inside the graph: right after the
+    loss, ``stopped`` = isnan(loss) is computed on the device (all-reduced with MAX over the ranks, on the main stream
+    before backward, so the flag's collective precedes every bucket's on every rank), and the Adam kernels read it when
+    they run: a replay with a NaN loss leaves weights, Adam moments and the step count untouched.  ``stopped`` is a
+    static one-element tensor next to ``loss`` and ``max_score``.  ``example_batch``: copied into the static batch before
+    the warm-up steps, so that they run on real data."""
+
+    def __init__(self, trainer, optimizer, batch_shape, warmup=3, bucket_mb=12.0, stop_on_nan=False,
+                 example_batch=None):
+        if stop_on_nan and not isinstance(optimizer, optim.Adam):
+            raise ValueError("GraphedTrainStep(stop_on_nan=True) needs cpc_b200.optim.Adam, whose kernels read the stop "
+                             "flag on the device; got %s" % type(optimizer).__name__)
         self.trainer, self.optimizer = trainer, optimizer
         self.world = trainer.world
+        self.stop_on_nan = stop_on_nan
         dev = trainer.device
         self.static_batch = torch.zeros(batch_shape, dtype=torch.float32, device=dev)
+        if example_batch is not None:
+            self.static_batch.copy_(example_batch)
         self.params = [p for p in trainer.model.parameters() if p.requires_grad]
         self.update_graph = None
         self.overlap_description = "single rank: no collective"
@@ -446,7 +502,7 @@ class GraphedTrainStep:
         if self.world == 1:
             optimizer.zero_grad(set_to_none=True)
             with torch.cuda.graph(self.graph):
-                self.loss, self.max_score = self._step_body()
+                self.loss, self.max_score, self.stopped = self._step_body()
             return
         # "thread_local": ProcessGroupNCCL's watchdog thread polls events of earlier (eager) collectives with
         # cudaEventQuery; under the default "global" capture mode such a call from ANY thread invalidates the capture
@@ -454,7 +510,7 @@ class GraphedTrainStep:
         torch.cuda.synchronize(dev)
         try:
             with torch.cuda.graph(self.graph, capture_error_mode="thread_local"):
-                self.loss, self.max_score = self._step_body()
+                self.loss, self.max_score, self.stopped = self._step_body()
             self.overlap_description = ("NCCL all-reduce of %d gradient buckets captured inside the step's CUDA graph on a "
                                         "communication stream forked from backward (bucket bytes: %s)"
                                         % (len(self.buckets), [4 * (hi - lo) for lo, hi, _ in self.buckets]))
@@ -504,31 +560,50 @@ class GraphedTrainStep:
         with torch.cuda.stream(self.comm_stream):
             torch.distributed.all_reduce(self.flat[lo:hi], op=torch.distributed.ReduceOp.SUM)
 
+    def _nan_flag(self, loss):
+        """(1,) fp32: 1 when the loss is NaN on any rank (trainer._any_rank_nan without the host read); None unless
+        stop_on_nan.  In the two-graph fallback the all-reduce runs eagerly between the graphs (``__call__``)."""
+        if not self.stop_on_nan:
+            return None
+        flag = torch.isnan(loss.detach()).to(torch.float32).reshape(1)
+        if self.world > 1 and not self._serial:
+            torch.distributed.all_reduce(flag, op=torch.distributed.ReduceOp.MAX)
+        return flag
+
     def _step_body(self):
-        """forward + backward (+ overlapped bucket all-reduces) + optimizer; identical eager (warm-up) and captured."""
+        """forward + backward (+ overlapped bucket all-reduces) + optimizer; identical eager (warm-up) and captured.
+        Returns (loss, max_score, stop flag or None)."""
         trainer, optimizer = self.trainer, self.optimizer
         if self.world == 1:
             optimizer.zero_grad(set_to_none=True)
             loss, max_score = trainer.loss_on_batch(self.static_batch)
+            flag = self._nan_flag(loss)
             loss.backward()
-            optimizer.step()
-            return loss.detach(), max_score.detach()
+            if flag is None:
+                optimizer.step()
+            else:
+                optimizer.step(skip_if=flag)
+            return loss.detach(), max_score.detach(), flag
         self.flat.zero_()                                        # gradients accumulate in place into the flat views
         self._pending = [len(ms) for _, _, ms in self.buckets]
         loss, max_score = trainer.loss_on_batch(self.static_batch)
+        flag = self._nan_flag(loss)
         loss.backward()
         if self._serial:
-            return loss.detach(), max_score.detach()
+            return loss.detach(), max_score.detach(), flag
         for i, left in enumerate(self._pending):                 # parameters that received no gradient this step
             if left > 0:
                 self._reduce_bucket(i)
         torch.cuda.current_stream(self.trainer.device).wait_stream(self.comm_stream)
-        self._optimizer_step()
-        return loss.detach(), max_score.detach()
+        self._optimizer_step(flag)
+        return loss.detach(), max_score.detach(), flag
 
-    def _optimizer_step(self):
+    def _optimizer_step(self, flag=None):
         if isinstance(self.optimizer, optim.Adam):               # reads the summed gradients in place, scaled by 1/W
-            self.optimizer.step(grad_scale=1.0 / self.world)
+            if flag is None:
+                self.optimizer.step(grad_scale=1.0 / self.world)
+            else:
+                self.optimizer.step(grad_scale=1.0 / self.world, skip_if=flag)
         else:
             self.flat.div_(self.world)
             self.optimizer.step()
@@ -538,10 +613,10 @@ class GraphedTrainStep:
         self._serial = True
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph, capture_error_mode="thread_local"):
-            self.loss, self.max_score = self._step_body()
+            self.loss, self.max_score, self.stopped = self._step_body()
         self.update_graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.update_graph, pool=self.graph.pool(), capture_error_mode="thread_local"):
-            self._optimizer_step()
+            self._optimizer_step(self.stopped)
         self.overlap_description = "not overlapped: two graphs around one eager NCCL all-reduce (capture failed: %s)" % why
 
     def remove_hooks(self):
@@ -554,6 +629,8 @@ class GraphedTrainStep:
         self.graph.replay()
         if self.update_graph is not None:
             torch.distributed.all_reduce(self.flat, op=torch.distributed.ReduceOp.SUM)
+            if self.stopped is not None:
+                torch.distributed.all_reduce(self.stopped, op=torch.distributed.ReduceOp.MAX)
             self.update_graph.replay()
         return self.loss, self.max_score
 

@@ -7,6 +7,8 @@
 //   p -= lr / (1 - beta1^t) * m / (sqrt(v) / sqrt(1 - beta2^t) + eps)
 // The step count t lives on the device (CUDA-graph replays advance it); the bias corrections are evaluated in
 // double precision by a one-thread kernel in front of the update.
+// An optional device flag `skip` is read by both kernels when they run: a non-zero flag turns the launch into a no-op
+// (parameters, moments, step count and bias corrections untouched), so a captured step can decide per replay.
 #include "common.cuh"
 
 namespace cpc {
@@ -25,7 +27,8 @@ struct AdamTable {
 };
 
 // state[0] = t (advanced here), state[1] = lr / (1 - beta1^t), state[2] = 1 / sqrt(1 - beta2^t)
-__global__ void adam_tick_kernel(float* state, double lr, double beta1, double beta2) {
+__global__ void adam_tick_kernel(float* state, const float* skip, double lr, double beta1, double beta2) {
+    if (skip && *skip != 0.f) return;
     const double t = (double)state[0] + 1.0;
     state[0] = (float)t;
     state[1] = (float)(lr / (1.0 - pow(beta1, t)));
@@ -47,7 +50,9 @@ __device__ __forceinline__ void adam_one(float& p, float g, float& m, float& v, 
 }
 
 __global__ void __launch_bounds__(256) adam_update_kernel(const __grid_constant__ AdamTable tab,
-                                                         const float* __restrict__ state, const AdamScalars a) {
+                                                         const float* __restrict__ state, const float* skip,
+                                                         const AdamScalars a) {
+    if (skip && *skip != 0.f) return;
     // which tensor does this block work on? (block_start is ascending; <= 48 entries in the constant bank)
     int lo = 0, hi = tab.count - 1;
     while (lo < hi) {
@@ -99,9 +104,9 @@ __global__ void __launch_bounds__(256) adam_update_kernel(const __grid_constant_
 
 using namespace cpc;
 
-extern "C" int cpc_adam_step(int32_t n_tensors, void* const* params, const void* const* grads, void* const* exp_avg,
-                             void* const* exp_avg_sq, const int64_t* numel, float* step_state,
-                             const cpc_adam_params* a, void* stream) {
+extern "C" int cpc_adam_step_ex(int32_t n_tensors, void* const* params, const void* const* grads, void* const* exp_avg,
+                                void* const* exp_avg_sq, const int64_t* numel, float* step_state, const float* skip,
+                                const cpc_adam_params* a, void* stream) {
     if (!a || !step_state || (n_tensors > 0 && (!params || !grads || !exp_avg || !exp_avg_sq || !numel))) return CPC_ERR_NULL;
     if (n_tensors < 0 || !(a->beta1 >= 0. && a->beta1 < 1.) || !(a->beta2 >= 0. && a->beta2 < 1.) || !(a->eps >= 0.))
         return CPC_ERR_BAD_SHAPE;
@@ -117,7 +122,7 @@ extern "C" int cpc_adam_step(int32_t n_tensors, void* const* params, const void*
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     const AdamScalars sc{(float)a->beta2, (float)(1.0 - a->beta1), (float)(1.0 - a->beta2), (float)a->eps,
                          (float)a->weight_decay, a->grad_scale, a->maximize};
-    adam_tick_kernel<<<1, 1, 0, s>>>(step_state, a->lr, a->beta1, a->beta2);
+    adam_tick_kernel<<<1, 1, 0, s>>>(step_state, skip, a->lr, a->beta1, a->beta2);
     CPC_LAUNCH_CHECK();
     count_launch();
     int i = 0;
@@ -139,9 +144,15 @@ extern "C" int cpc_adam_step(int32_t n_tensors, void* const* params, const void*
         }
         if (tab.count == 0) break;
         tab.block_start[tab.count] = blocks;
-        adam_update_kernel<<<blocks, 256, 0, s>>>(tab, step_state, sc);
+        adam_update_kernel<<<blocks, 256, 0, s>>>(tab, step_state, skip, sc);
         CPC_LAUNCH_CHECK();
         count_launch();
     }
     return CPC_OK;
+}
+
+extern "C" int cpc_adam_step(int32_t n_tensors, void* const* params, const void* const* grads, void* const* exp_avg,
+                             void* const* exp_avg_sq, const int64_t* numel, float* step_state,
+                             const cpc_adam_params* a, void* stream) {
+    return cpc_adam_step_ex(n_tensors, params, grads, exp_avg, exp_avg_sq, numel, step_state, nullptr, a, stream);
 }

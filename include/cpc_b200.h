@@ -381,6 +381,15 @@ int cpc_adam_step(int32_t n_tensors, void* const* params, const void* const* gra
                   void* const* exp_avg_sq, const int64_t* numel, float* step_state,
                   const cpc_adam_params* p, void* stream);
 
+/* cpc_adam_step with a guard: skip is NULL (always update) or a device pointer to one float that both kernels read
+ * when they execute, not when they are enqueued.  *skip != 0 makes the call change nothing: not the parameters, not
+ * exp_avg / exp_avg_sq, not step_state.  A captured graph holding this call therefore decides per replay whether
+ * the step applies (ContrastiveEstimationTrainer.train(cuda_graph=True) stops on a NaN loss this way).  Arguments are
+ * validated as for cpc_adam_step, before the device is touched; cpc_adam_step is this call with skip = NULL. */
+int cpc_adam_step_ex(int32_t n_tensors, void* const* params, const void* const* grads, void* const* exp_avg,
+                     void* const* exp_avg_sq, const int64_t* numel, float* step_state, const float* skip,
+                     const cpc_adam_params* p, void* stream);
+
 /* ------------------------------------------------------------------------------------------------
  * 6. Batch assembly from raw PCM WAV bytes (the input path of AudioDataset, audio_dataset.py:61-113).
  *    The host copies the bytes of whole interleaved frames; one kernel decodes the first channel of each and writes
